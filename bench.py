@@ -21,7 +21,9 @@ Rank 0 prints ONE JSON line:
              objects) + the restated CTC (the reference has no CPU CTC) on a bounded sample, N=1 only
   gpu_reference  the reference's own gpucompute kernels (oracle/_ref/ref_dump_gpu) on the same GPU and batch, N=1 only
   replicas_identical  (N > 1) sha256 of every rank's parameters after the timed steps agree
---impl reference times the CPU arm as the main line, on the full minibatch (at most 2 timed steps are executed).
+--dump-outputs DIR writes what the last timed step returned on rank 0 as DIR/<name>.npy (see dump_outputs); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
+--impl reference times the CPU arm as the main line, on the full minibatch (tens of seconds per step on the host).
 """
 from __future__ import annotations
 
@@ -44,7 +46,6 @@ from eesen_b200 import kaldi_io, synth  # noqa: E402
 METRIC = "ctc_train_frames_per_sec"
 UNIT = "frames/s"
 REF_SAMPLE_UTTS = 8  # bounded CPU sample inside the GPU arm's line: this many utterances of the same workload per step
-REF_MAX_STEPS = 2    # --impl reference: full minibatch, at most this many timed steps (tens of seconds each)
 
 
 def load_peaks():
@@ -178,9 +179,9 @@ def run_reference_impl(args, w):
     if rank != 0:
         return 0
     # the SAME configuration as the GPU arm: the full w.S-utterance minibatch per step.  One such step takes the
-    # host cores tens of seconds, so at most REF_MAX_STEPS timed steps (after at most one warm-up step) are
-    # executed whatever --steps / --warmup ask for; `sample` says how many were.
-    run_steps, run_warm = min(args.steps, REF_MAX_STEPS), min(args.warmup, 1)
+    # host cores tens of seconds, so at most one warm-up step is executed whatever --warmup asks for; `sample` says
+    # how many were.  --steps timed steps are executed.
+    run_steps, run_warm = args.steps, min(args.warmup, 1)
     with tempfile.TemporaryDirectory() as tmp:
         cb = cpu_reference_arm(w, run_steps, run_warm, tmp, sample_utts=args.ref_utts or w.S)
     cb["sample"] += f"; {run_steps} timed step(s) after {run_warm} warm-up executed of --steps {args.steps} --warmup {args.warmup}"
@@ -222,6 +223,43 @@ def gpu_reference_leg(w, tmp: str, steps: int = 2):
 
 
 # --------------------------------------------------------------------------------------- GPU arm
+DUMP_SAMPLE = 1 << 20   # momentum buffers: this many entries at fixed, seeded positions
+DUMP_LIMIT = 63_000_000  # bytes of all dumped arrays together: with the .npy headers under 64 MB however counted
+
+
+def seeded_sample(a, n, seed):
+    """n entries of a (flattened) at fixed positions drawn from `seed`, in order; all of a if it has no more."""
+    a = a.ravel()
+    if a.size <= n:
+        return a
+    return a[np.sort(np.random.default_rng(seed).choice(a.size, n, replace=False))]
+
+
+def last_step_outputs(net, n_layers, stats):
+    """What a caller of the timed path holds after its last step: the statistics, log p(z|x) per utterance, the
+    posteriors and the CTC gradient [T*S x K], the updated parameters and a fixed, seeded sample of the momentum
+    buffers.  When the parameters, posteriors and gradient together would take the dump past DUMP_LIMIT (C4: 27.5 M
+    parameters), each of the three is replaced by a fixed, seeded sample of its share of what is left (names
+    <name>_sample); C2 is dumped whole, about 50 MB."""
+    out = {"stats": np.array([stats[k] for k in ("obj", "token_err", "ref_tokens", "frames")], np.float64),
+           "pzx": net.get(101).ravel(), "momentum_sample": seeded_sample(net.corr(), DUMP_SAMPLE, 0)}
+    big = {"posteriors": net.get(n_layers), "obj_diff": net.get(100), "params": net.params()}
+    room = DUMP_LIMIT - sum(v.nbytes for v in out.values())
+    total = sum(v.nbytes for v in big.values())
+    for seed, (k, v) in enumerate(big.items(), 1):
+        if total <= room:
+            out[k] = v
+        else:
+            out[k + "_sample"] = seeded_sample(v, room * v.size // total, seed)
+    return out
+
+
+def dump_outputs(outdir: str, outputs) -> None:
+    os.makedirs(outdir, exist_ok=True)
+    for k, v in outputs.items():
+        np.save(os.path.join(outdir, k + ".npy"), np.ascontiguousarray(v))
+
+
 def rooflines_from_profile(ms, counts, w, batches, peaks, steps, prec, wall_ms, engines=(1, 1)):
     """Per-kernel rooflines from the library's per-launch CUDA events (eesen_b200_profile).
     Algorithmic figures (DESIGN.md section 4; SURVEY.md section 8d split by kernel):
@@ -310,7 +348,8 @@ def run_ours(args, w):
 
     tmp = tempfile.mkdtemp(prefix="eesen_b200_bench_")
     model_path = os.path.join(tmp, f"model_{rank}")
-    kaldi_io.write_model(model_path, synth.make_model(w, seed=0))  # identical weights on every rank
+    spec = synth.make_model(w, seed=0)
+    kaldi_io.write_model(model_path, spec)  # identical weights on every rank
     net = binding.Net(ctx, model_path)
     net.set_train_options(w.learn_rate, w.momentum)
 
@@ -356,6 +395,8 @@ def run_ours(args, w):
     launches = ctx.launches - l0
     clocks = sampler.stop() if rank == 0 else None
     frames_dev = sum(pool[i % len(pool)].valid_frames for i in range(args.steps))
+    # read before the e2e and TF32 passes below train the model further
+    outputs = last_step_outputs(net, len(spec.layers), stats) if args.dump_outputs and rank == 0 else None
     padded_dev = sum(pool[i % len(pool)].feats.shape[0] for i in range(args.steps))
 
     # ---- timed region 2: end to end through the public call with HOST buffers.  The packed features of every
@@ -476,6 +517,8 @@ def run_ours(args, w):
         if world == 1 and not args.no_gpu_reference:
             # the context must not hold the GPU's memory hostage while the reference allocates its ~3 GB
             line["gpu_reference"] = gpu_reference_leg(w, tmp)
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     net.close()
     ctx.close()
@@ -498,7 +541,11 @@ def main():
     ap.add_argument("--no-alt", action="store_true", help="skip the informational TF32 pass")
     ap.add_argument("--no-gpu-reference", action="store_true", help="skip timing the reference's own gpucompute kernels")
     ap.add_argument("--ref-utts", type=int, default=0, help="--impl reference: utterances per step (default: the full minibatch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours (the CPU arm returns no device outputs)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     w = synth.WORKLOADS[args.workload]
     if args.impl == "reference":

@@ -301,13 +301,25 @@ def net_output(on: "OracleNet", feats, frames, apply_log=False, log_priors=None,
     return y
 
 
+# Every call of a binary under oracle/_ref goes through RUNNER (same signature as subprocess.run with
+# capture_output=True, text=True).  The tests set it to replay the runs stored under tests/golden/runs, so they do
+# not need the reference's sources (tests/util.py:stored_runs).
+RUNNER = None
+
+
+def _run(cmd: List[str], env=None, timeout: Optional[int] = None):
+    if RUNNER is not None:
+        return RUNNER(cmd, env=env, timeout=timeout)
+    return subprocess.run(cmd, capture_output=True, text=True, env=env, timeout=timeout)
+
+
 def run_reference_tool(tool: str, args: List[str], timeout: int = 600, threads: Optional[int] = None):
-    """Run one of the reference's own command-line tools built under oracle/_ref (CPU build)."""
+    """Run one of the reference's own command-line tools built under oracle/_ref."""
     exe = os.path.join(REFDIR, tool)
     env = dict(os.environ)
     if threads is not None:
         env["OPENBLAS_NUM_THREADS"] = str(threads)
-    r = subprocess.run([exe] + list(args), capture_output=True, text=True, env=env, timeout=timeout)
+    r = _run([exe] + list(args), env=env, timeout=timeout)
     if r.returncode != 0:
         raise RuntimeError(f"{tool} failed ({r.returncode}):\n{r.stdout[-2000:]}\n{r.stderr[-4000:]}")
     return r
@@ -360,7 +372,7 @@ def run_reference(kind: str, model_path: str, batch_path: str, outdir: str, lr: 
     env = dict(os.environ)
     if threads is not None:
         env["OPENBLAS_NUM_THREADS"] = str(threads)
-    r = subprocess.run(cmd, capture_output=True, text=True, env=env, timeout=timeout)
+    r = _run(cmd, env=env, timeout=timeout)
     if r.returncode != 0:
         raise RuntimeError(f"reference run failed ({r.returncode}):\n{r.stdout[-2000:]}\n{r.stderr[-4000:]}")
     info = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])

@@ -20,6 +20,17 @@ minted from runs of the reference itself on seeded synthetic inputs:
   reference writes into the model (<BiLstmAccus>/<AffineAccus>).
 
 Inputs are regenerated from (workload, seeds) by eesen_b200.synth, so only outputs are stored.
+
+``runs/<name>.npz`` hold the runs of the reference binaries the tests make themselves (tests/util.py:stored_runs).
+The tests write them, with the reference built under oracle/_ref; these two commands select exactly those tests:
+
+    EESEN_B200_RECORD_RUNS=1 python -m pytest tests -m "not gpu" \
+        -k "reference_reads_and_rewrites or net_initialize or reference_driver_reads or live or token_error_count"
+    EESEN_B200_RECORD_RUNS=1 python -m pytest tests -m gpu -k "gpucompute or format_to_nonparallel_and_extract"  # B200
+
+The dropout fixtures (runs/tiny_drop_*) change with every recording: the reference draws its masks from a
+random_device-seeded generator, and the fixture stores the masks it drew.  So does runs/net_initialize (unseeded
+initialisation); the stored stdout / stderr carry timings.  Everything else records bit for bit the same.
 """
 import os
 import sys

@@ -9,7 +9,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from util import ROOT, case
+from util import ROOT, case, stored_runs
 from eesen_b200 import binding, kaldi_io, synth
 
 HEADER = os.path.join(ROOT, "include", "eesen_b200.h")
@@ -101,8 +101,6 @@ def test_model_accumulators_roundtrip():
     assert np.array_equal(net.flat_accus(), net2.flat_accus())
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_dump_cpu")),
-                    reason="reference build (oracle/_ref) not present")
 def test_reference_reads_and_rewrites_our_accumulators():
     """The reference's Net::Read accepts the accumulator blocks we write and its Net::Write puts them back
     byte for byte (SGD leaves them alone), so the two writers agree on the format."""
@@ -117,15 +115,15 @@ def test_reference_reads_and_rewrites_our_accumulators():
         kaldi_io.write_batch_file(d + "/batch.bin", b)
         diff = np.zeros((b.feats.shape[0], w.classes), np.float32)
         np.save(d + "/diff.npy", diff)
-        oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", 0.0, 0.0, steps=1,
-                             diff_in=d + "/diff.npy")
+        with stored_runs("tiny_accus_rewrite", d, keep=("out/model_out",)):
+            oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", 0.0, 0.0, steps=1,
+                                 diff_in=d + "/diff.npy")
         assert open(d + "/out/model_out", "rb").read() == open(d + "/model", "rb").read()
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_net_initialize")),
-                    reason="reference net-initialize not built")
 def test_reads_model_written_by_reference_net_initialize():
     """Byte-compatibility with the reference's own model factory (src/netbin/net-initialize.cc)."""
+    from oracle import oracle
     with tempfile.TemporaryDirectory() as d:
         proto = os.path.join(d, "proto")
         with open(proto, "w") as f:
@@ -133,8 +131,8 @@ def test_reads_model_written_by_reference_net_initialize():
                     "<AffineTransform> <InputDim> 32 <OutputDim> 6 <ParamRange> 0.1\n"
                     "<Softmax> <InputDim> 6 <OutputDim> 6\n</Nnet>\n")
         out = os.path.join(d, "nnet.init")
-        exe = os.path.join(ROOT, "oracle", "_ref", "ref_net_initialize")
-        r = subprocess.run([exe, "--binary=true", proto, out], capture_output=True, text=True)
+        with stored_runs("net_initialize", d, sample=False):
+            r = oracle.run_reference_tool("ref_net_initialize", ["--binary=true", proto, out])
         assert r.returncode == 0, r.stderr[-2000:]
         net = kaldi_io.read_model(out)
         assert [l.kind for l in net.layers] == ["bilstm", "affine", "softmax"]
@@ -179,14 +177,11 @@ def test_feature_and_label_archives(tmp_path):
     assert open(tmp_path / "l.ark").read() == "utt1 1 2\nutt2 3\n"
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_train_ctc_parallel")),
-                    reason="reference train-ctc-parallel (CPU build) not built")
 def test_reference_driver_reads_our_archives_and_reports_the_same_accuracy():
     """The reference's own driver (CPU build, --cross-validate: forward + ErrorRateMSeq only) on the feature / label
     archives and the model our writers produce: it must read them, skip what it skips (an utterance without
     targets, one above --frame-limit) and print the TOKEN_ACCURACY the restatement computes for the rest."""
     import re
-    import subprocess
     from oracle import oracle
     w, net, b = case("small", 5, 6)
     for l in net.layers:
@@ -203,10 +198,11 @@ def test_reference_driver_reads_our_archives_and_reports_the_same_accuracy():
         kaldi_io.write_feature_ark(d + "/feats.ark", keys, utts)
         kaldi_io.write_label_ark(d + "/labels.ark", [k for i, k in enumerate(keys) if i != no_target],
                                  [l for i, l in enumerate(labels) if i != no_target])
-        exe = os.path.join(ROOT, "oracle", "_ref", "ref_train_ctc_parallel")
-        r = subprocess.run([exe, "--cross-validate=true", "--num-sequence=3", f"--frame-limit={limit}", "--report-step=1000",
-                            f"ark:{d}/feats.ark", f"ark,t:{d}/labels.ark", d + "/model"], capture_output=True, text=True,
-                           timeout=600, env=dict(os.environ, OPENBLAS_NUM_THREADS="4"))
+        with stored_runs("small_reference_driver_cross_validate", d):
+            r = oracle.run_reference_tool("ref_train_ctc_parallel",
+                                          ["--cross-validate=true", "--num-sequence=3", f"--frame-limit={limit}",
+                                           "--report-step=1000", f"ark:{d}/feats.ark", f"ark,t:{d}/labels.ark", d + "/model"],
+                                          timeout=600, threads=4)
     assert r.returncode == 0, r.stderr[-3000:]
     log = r.stdout + r.stderr
     acc = float(re.search(r"TOKEN_ACCURACY >> ([-0-9.e+]+)% <<", log).group(1))

@@ -7,7 +7,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from util import GOLDEN, assert_close, case, golden_arrays
+from util import GOLDEN, assert_close, case, golden_arrays, stored_runs
 from eesen_b200 import kaldi_io
 from oracle import oracle
 
@@ -69,7 +69,6 @@ def check_mask_statistics(masks, net):
             assert np.all(m["rmask"] == m["rmask"][0])
 
 
-@pytest.mark.skipif(not oracle.have_reference("cpu"), reason="reference build (oracle/_ref) not present")
 @pytest.mark.parametrize("variant", sorted(VARIANTS))
 def test_oracle_dropout_matches_reference_cpu_live(variant):
     w, net, b = drop_case("tiny", variant)
@@ -81,7 +80,10 @@ def test_oracle_dropout_matches_reference_cpu_live(variant):
         rows_pad = np.concatenate([np.arange(b.frames[s], b.T) * b.S + s for s in range(b.S)])
         diff[rows_pad.astype(np.int64)] = 0.0          # CTC never produces gradient on padding frames
         np.save(d + "/diff.npy", diff)
-        oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=1, diff_in=d + "/diff.npy")
+        with stored_runs(f"tiny_drop_{variant.replace('+', '_')}_cpu", d, whole=("out/mask_*",),
+                         keep=("out/out_l[1-9].npy", "out/in_diff.npy", "out/grad_*", "out/mask_*", "out/model_out")):
+            oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=1,
+                                 diff_in=d + "/diff.npy")
         dump = oracle.load_dump(d + "/out")
         m2 = kaldi_io.read_model(d + "/out/model_out")
     masks = masks_from_dump(dump, net, b)
@@ -90,10 +92,10 @@ def test_oracle_dropout_matches_reference_cpu_live(variant):
     on = oracle.OracleNet(net, np.float32)
     r = on.train_step(b, lr, mom, diff_override=diff, masks=masks)
     for i in range(1, len(net.layers) + 1):
-        assert_close(f"out_l{i}", on.acts[i], dump[f"out_l{i}"], atol=2e-6)
-    assert_close("in_diff", r["in_diff"], dump["in_diff"], atol=1e-6, rtol=1e-4)
-    assert_close("corr", on.flat_corr(), golden_arrays(dump, net), atol=2e-5, rtol=1e-4)
-    assert_close("params", on.flat_params(), m2.flat_params(), atol=1e-6)
+        assert_close(f"out_l{i}", on.acts[i], dump[f"out_l{i}"], atol=2e-6, stored=True)
+    assert_close("in_diff", r["in_diff"], dump["in_diff"], atol=1e-6, rtol=1e-4, stored=True)
+    assert_close("corr", on.flat_corr(), golden_arrays(dump, net), atol=2e-5, rtol=1e-4, stored=True)
+    assert_close("params", on.flat_params(), m2.flat_params(), atol=1e-6, stored=True)
     assert m2.layers[0].dropout == net.layers[0].dropout or all(
         abs(float(m2.layers[0].dropout.get(k, 0)) - float(v)) < 1e-7 for k, v in net.layers[0].dropout.items())
 

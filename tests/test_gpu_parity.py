@@ -1,7 +1,7 @@
 """GPU parity tests (run with -m gpu on the B200 box).  Everything goes through the C ABI
 (include/eesen_b200.h) via eesen_b200.binding; the checker is the oracle (oracle/), the committed
-golden vectors minted from the reference, and -- live on the box -- the reference's own gpucompute
-build (oracle/_ref/ref_dump_gpu, compiled from the unmodified sources for sm_100a).
+golden vectors minted from the reference, and stored runs of the reference's own gpucompute build
+(oracle/_ref/ref_dump_gpu, compiled from the unmodified sources for sm_100a; tests/util.py:stored_runs).
 
 Stated tolerances (fp32 storage everywhere):
   default arithmetic "fp32x3" (3xTF32 split, fp32 accumulate): fp32-faithful
@@ -19,7 +19,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from util import GOLDEN, assert_close, case, golden_arrays, model_file
+from util import GOLDEN, assert_close, case, golden_arrays, model_file, stored_runs
 from eesen_b200 import binding, kaldi_io, synth
 from oracle import oracle
 
@@ -360,7 +360,15 @@ def test_train_step_vs_reference_golden(ctx, wl, kind):
     n.close()
 
 
-@pytest.mark.skipif(not oracle.have_reference("gpu"), reason="oracle/_ref/ref_dump_gpu not built")
+# what the comparisons with ref_dump_gpu read of its output directory, and the cells the stored runs keep of each
+# compared tensor (spread over every utterance and every weight matrix; the momentum buffers, grad_*, count as one).
+# log p(z|x) is kept whole.
+REF_STEP_OUTPUTS = ("out/pzx.npy", "out/net_out.npy", "out/obj_diff.npy", "out/in_diff.npy", "out/grad_*", "out/model_out")
+REF_STEP_CELLS = {"small": 1024, "mid": 2048}
+REF_FULL_SIZE_OUTPUTS = ("out/pzx.npy", "out/net_out.npy", "out/obj_diff.npy", "out/model_out")
+REF_FULL_SIZE_CELLS = {"out/net_out.npy": 3072, "out/obj_diff.npy": 3072, "out/model_out": 3072}
+
+
 @pytest.mark.parametrize("wl,steps", [("small", 2), ("mid", 1)])
 def test_train_step_vs_reference_gpucompute_live(ctx, wl, steps):
     """Same inputs through the reference's own gpucompute kernels (compiled for sm_100a) on this GPU."""
@@ -369,16 +377,18 @@ def test_train_step_vs_reference_gpucompute_live(ctx, wl, steps):
     d = tempfile.mkdtemp()
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
-    oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=steps)
+    with stored_runs(f"{wl}_gpucompute_{steps}steps", d, keep=REF_STEP_OUTPUTS, whole=("out/pzx.npy",),
+                     cells={p: REF_STEP_CELLS[wl] for p in REF_STEP_OUTPUTS[1:]}):
+        oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=steps)
     ref = oracle.load_dump(d + "/out")
     n, st = _gpu_steps(ctx, net, b, lr, mom, steps)
     assert_close("pzx", n.get(101).ravel(), ref["pzx"], atol=0, rtol=2e-5)      # north_star: 1e-4 relative
-    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=2e-5)
-    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=diff_atol(ref["pzx"]))
-    assert_close("in_diff", n.get(102), ref["in_diff"], atol=2e-5, rtol=1e-3)
-    assert_close("corr", n.corr(), golden_arrays(ref, net), atol=2e-3, rtol=2e-3)
+    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=2e-5, stored=True)
+    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=diff_atol(ref["pzx"]), stored=True)
+    assert_close("in_diff", n.get(102), ref["in_diff"], atol=2e-5, rtol=1e-3, stored=True)
+    assert_close("corr", n.corr(), golden_arrays(ref, net), atol=2e-3, rtol=2e-3, stored=True)
     m2 = kaldi_io.read_model(d + "/out/model_out")
-    assert_close("params", n.params(), m2.flat_params(), atol=5e-6)
+    assert_close("params", n.params(), m2.flat_params(), atol=5e-6, stored=True)
     n.close()
 
 
@@ -423,7 +433,6 @@ def test_lstm_parallel_vs_reference_golden(ctx, wl):
     n.close()
 
 
-@pytest.mark.skipif(not oracle.have_reference("gpu"), reason="oracle/_ref/ref_dump_gpu not built")
 def test_lstm_parallel_vs_reference_gpucompute_live_and_model_bytes(ctx):
     """Live against the reference's GPU build with Adagrad, incl. the model file.  The reference stores the
     WEIGHTS a second time under <LstmAccus> (lstm-layer.h:153-163, a bug: a reloaded model then takes
@@ -433,16 +442,17 @@ def test_lstm_parallel_vs_reference_gpucompute_live_and_model_bytes(ctx):
     d = tempfile.mkdtemp()
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
-    oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=2, opt="Adagrad")
+    with stored_runs("small_uni_gpucompute_adagrad", d, keep=("out/model_out",)):
+        oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=2, opt="Adagrad")
     m2 = kaldi_io.read_model(d + "/out/model_out")
     n = _adaptive_steps(ctx, net, b, lr, mom, "Adagrad", 2)
-    assert_close("params", n.params(), m2.flat_params(), atol=_ada_atol(lr))
+    assert_close("params", n.params(), m2.flat_params(), atol=_ada_atol(lr), stored=True)
     n.write(d + "/ours_out", True)
     ours = kaldi_io.read_model(d + "/ours_out")
     for lo, lt in zip(ours.layers, m2.layers):
         if lo.kind == "lstm":
             for k in lo.param_names():      # theirs: <LstmAccus> block == the weights block; ours: the accumulators
-                assert np.array_equal(lt.accus[k], lt.params[k])
+                assert np.array_equal(lt.accus[k], lt.params[k], equal_nan=True)
                 assert lo.accus[k].shape == lo.params[k].shape and (lo.accus[k] >= 0).all()
             assert any(not np.array_equal(lo.accus[k], lo.params[k]) for k in lo.param_names())
     assert len(open(d + "/ours_out", "rb").read()) == len(open(d + "/out/model_out", "rb").read())
@@ -539,7 +549,6 @@ def test_adaptive_update_vs_reference_golden(ctx, wl, opt):
     n.close()
 
 
-@pytest.mark.skipif(not oracle.have_reference("gpu"), reason="oracle/_ref/ref_dump_gpu not built")
 @pytest.mark.parametrize("opt", ["Adagrad", "RMSProp"])
 def test_adaptive_update_vs_reference_gpucompute_live(ctx, opt):
     w, net, b = case("small", 21, 22)
@@ -547,11 +556,12 @@ def test_adaptive_update_vs_reference_gpucompute_live(ctx, opt):
     d = tempfile.mkdtemp()
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
-    oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=3, opt=opt)
+    with stored_runs(f"small_gpucompute_{opt.lower()}", d, keep=("out/model_out",)):
+        oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, steps=3, opt=opt)
     m2 = kaldi_io.read_model(d + "/out/model_out")
     n = _adaptive_steps(ctx, net, b, lr, mom, opt, 3)
-    assert_close("accu", n.accu(), m2.flat_accus(), atol=1e-7, rtol=5e-3)
-    assert_close("params", n.params(), m2.flat_params(), atol=_ada_atol(lr))
+    assert_close("accu", n.accu(), m2.flat_accus(), atol=1e-7, rtol=5e-3, stored=True)
+    assert_close("params", n.params(), m2.flat_params(), atol=_ada_atol(lr), stored=True)
     # the model we write carries the accumulators where the reference puts them: the reference's own
     # writer and ours agree token for token (same length, same tokens; payload compared above)
     out = d + "/ours_out"
@@ -687,7 +697,6 @@ def test_c2_stream_knobs_give_the_same_step(ctx, c2_run, monkeypatch):
         c2.close()
 
 
-@pytest.mark.skipif(not oracle.have_reference("gpu"), reason="oracle/_ref/ref_dump_gpu not built")
 def test_c2_full_size_vs_reference_gpucompute(ctx):
     """BASELINE configs[1] at full size against the reference's own gpucompute run on the same inputs:
     CTC log-prob within 1e-4 relative (north_star) and per-frame gradients within the stated tolerance."""
@@ -697,22 +706,23 @@ def test_c2_full_size_vs_reference_gpucompute(ctx):
     d = tempfile.mkdtemp()
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
-    info = oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", w.learn_rate, w.momentum, steps=1)
+    with stored_runs("c2_gpucompute", d, keep=REF_FULL_SIZE_OUTPUTS, whole=("out/pzx.npy",), cells=REF_FULL_SIZE_CELLS):
+        oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", w.learn_rate, w.momentum, steps=1,
+                             dump_layers=False)      # the layer outputs are not compared here
     ref = oracle.load_dump(d + "/out")
     n, st = _gpu_steps(ctx, net, b, w.learn_rate, w.momentum, 1, want_in_diff=False)
     pzx = n.get(101).ravel()
     rel = np.abs(pzx - ref["pzx"]) / np.abs(ref["pzx"])
     assert rel.max() < 2e-5, rel.max()
-    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=5e-5)
-    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=2 * diff_atol(ref["pzx"]))
+    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=5e-5, stored=True)
+    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=2 * diff_atol(ref["pzx"]), stored=True)
     m2 = kaldi_io.read_model(d + "/out/model_out")
     # parameter update = lr * (momentum buffer); the buffers are sums over all T*S rows of per-frame
     # gradients that individually agree only to diff_atol (fp32 log-domain CTC at |log p| ~ 2000 in BOTH
     # implementations), so their difference random-walks to ~sqrt(T*S) * diff_atol
     rows = b.feats.shape[0]
     assert_close("params", n.params(), m2.flat_params(),
-                 atol=5e-6 + w.learn_rate * np.sqrt(rows) * diff_atol(ref["pzx"]))
-    print(f"reference gpucompute on this GPU: {info['valid_fps']:.0f} valid frames/s (one cold step)")
+                 atol=5e-6 + w.learn_rate * np.sqrt(rows) * diff_atol(ref["pzx"]), stored=True)
     n.close()
 
 
@@ -762,7 +772,6 @@ def c4_inputs():
     return w, synth.make_model(w, seed=0), synth.make_batch(w, seed=4)
 
 
-@pytest.mark.skipif(not oracle.have_reference("gpu"), reason="oracle/_ref/ref_dump_gpu not built")
 def test_c4_vs_reference_gpucompute_at_the_reference_row_limit(ctx):
     """BASELINE configs[3] (5x512 BiLSTM, K = 32, 64 utterances) against the reference's own gpucompute.  The
     reference CANNOT run the config at its full 2000 frames: CuVectorBase::AddColSumMat launches a grid of
@@ -776,19 +785,21 @@ def test_c4_vs_reference_gpucompute_at_the_reference_row_limit(ctx):
     d = tempfile.mkdtemp()
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
-    info = oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", w.learn_rate, w.momentum, steps=1,
-                                dump_layers=False)          # 1.3 GB of layer outputs are not needed here
+    with stored_runs("c4_t1000_gpucompute", d, keep=REF_FULL_SIZE_OUTPUTS, whole=("out/pzx.npy",),
+                     cells=REF_FULL_SIZE_CELLS):
+        oracle.run_reference("gpu", d + "/model", d + "/batch.bin", d + "/out", w.learn_rate, w.momentum, steps=1,
+                             dump_layers=False)      # 1.3 GB of layer outputs are not needed here
     ref = {k: np.load(os.path.join(d, "out", k + ".npy")) for k in ("pzx", "net_out", "obj_diff")}
     n, st = _gpu_steps(ctx, net, b, w.learn_rate, w.momentum, 1, want_in_diff=False)
     pzx = n.get(101).ravel()
     rel = np.abs(pzx - ref["pzx"]) / np.abs(ref["pzx"])
     assert rel.max() < 1e-4, rel.max()                       # north_star: CTC log-prob within 1e-4 relative
-    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=1e-4)
-    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=4 * diff_atol(ref["pzx"]))
+    assert_close("net_out", n.get(len(net.layers)), ref["net_out"], atol=1e-4, stored=True)
+    assert_close("obj_diff", n.get(100), ref["obj_diff"], atol=4 * diff_atol(ref["pzx"]), stored=True)
     m2 = kaldi_io.read_model(d + "/out/model_out")
     rows = b.feats.shape[0]
-    assert_close("params", n.params(), m2.flat_params(), atol=5e-6 + w.learn_rate * np.sqrt(rows) * 4 * diff_atol(ref["pzx"]))
-    print(f"reference gpucompute on this GPU, C4 at T=1000: {info['valid_fps']:.0f} valid frames/s (one cold step)")
+    assert_close("params", n.params(), m2.flat_params(), atol=5e-6 + w.learn_rate * np.sqrt(rows) * 4 * diff_atol(ref["pzx"]),
+                 stored=True)
     n.close()
 
 

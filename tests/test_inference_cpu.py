@@ -1,18 +1,15 @@
 """CPU tests of the forward-only path (SURVEY.md 8f N2): pin the restatement of
 net-output-extract (Net::Feedforward + ApplyLog + ClassPrior) against the reference's own CPU tool,
-live when oracle/_ref is present and through the committed fixture otherwise."""
+through stored runs of that tool and through the committed fixture."""
 import os
 import tempfile
 
 import numpy as np
 import pytest
 
-from util import GOLDEN, ROOT, assert_close, case
+from util import GOLDEN, assert_close, case, stored_runs
 from eesen_b200 import binding, kaldi_io, synth
 from oracle import oracle
-
-HAVE_TOOL = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "ref_net_output_extract"))
-
 
 def infer_case(wl="small", mseed=3, bseed=9):
     """Model + ragged utterances + class counts (one class below the cutoff) for the inference tests."""
@@ -36,11 +33,11 @@ def test_class_log_priors_restatement_vs_abi():
         assert_close("log priors", got[~big], a[~big], atol=1e-6)
 
 
-@pytest.mark.skipif(not HAVE_TOOL, reason="reference net-output-extract not built (oracle/_ref)")
 @pytest.mark.parametrize("nonparallel", [False, True])
 def test_oracle_matches_reference_net_output_extract_live(nonparallel):
     w, net, b, utts, counts = infer_case()
-    with tempfile.TemporaryDirectory() as d:
+    with tempfile.TemporaryDirectory() as d, \
+            stored_runs(f"small_net_output_extract{'_nonparallel' if nonparallel else ''}", d, sample=False):
         kaldi_io.write_model(d + "/model", net)
         model = d + "/model"
         if nonparallel:

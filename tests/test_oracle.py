@@ -3,7 +3,7 @@
 1. against the committed golden vectors minted from the UNMODIFIED reference (tests/golden, see
    make_golden.py) -- CPU build for BiLSTM/affine/softmax/SGD, GPU build (when the fixture exists)
    for the CTC alpha/beta/pzx/diff the reference only computes on a GPU;
-2. live against oracle/_ref/ref_dump_cpu when the reference build is present (this container);
+2. against stored runs of oracle/_ref/ref_dump_cpu (tests/util.py:stored_runs);
 3. CTC against torch.nn.functional.ctc_loss in fp64 (independent third opinion, SURVEY.md 8c);
 4. structural properties of the restatement itself.
 """
@@ -13,7 +13,7 @@ import tempfile
 import numpy as np
 import pytest
 
-from util import GOLDEN, assert_close, case, golden_arrays
+from util import GOLDEN, assert_close, case, golden_arrays, stored_runs
 from eesen_b200 import kaldi_io, synth
 from oracle import oracle
 
@@ -137,7 +137,11 @@ def test_oracle_adaptive_rules_closed_form():
         assert np.allclose(w, w0 - 0.01 * cc / np.sqrt(aa + 1e-6), rtol=1e-14)
 
 
-@pytest.mark.skipif(not oracle.have_reference("cpu"), reason="reference build (oracle/_ref) not present")
+def onehot_argmax(y):
+    """what the greedy token count reads of the posteriors: each row's argmax"""
+    return np.eye(y.shape[1], dtype=y.dtype)[y.argmax(1)]
+
+
 def test_oracle_matches_reference_cpu_live():
     w, net, b = case("small", 11, 12)
     lr, mom = 2e-3, 0.5
@@ -147,20 +151,21 @@ def test_oracle_matches_reference_cpu_live():
     kaldi_io.write_model(d + "/model", net)
     kaldi_io.write_batch_file(d + "/batch.bin", b)
     np.save(d + "/diff.npy", r["obj_diff"].astype(np.float32))
-    info = oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, diff_in=d + "/diff.npy")
+    with stored_runs("small_cpu_step", d, keep=("out/out_l[1-9].npy", "out/in_diff.npy", "out/grad_*", "out/net_out.npy",
+                                                "out/model_out"), transform={"out/net_out.npy": onehot_argmax}):
+        info = oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", lr, mom, diff_in=d + "/diff.npy")
     ref = oracle.load_dump(d + "/out")
     # Ctc::ErrorRateMSeq (greedy path, collapse, Levenshtein: ctc-loss.cc:235-298) runs on the CPU build too
     err, nref = oracle.greedy_token_errors(ref["net_out"], b.frames, b.labels, b.S)
     assert (float(info["token_err"]), int(info["ref_tokens"])) == (float(err), int(nref))
     for i in range(1, len(net.layers) + 1):
-        assert_close(f"out_l{i}", on.acts[i], ref[f"out_l{i}"], atol=2e-6)
-    assert_close("in_diff", r["in_diff"], ref["in_diff"], atol=1e-6, rtol=1e-4)
-    assert_close("corr", on.flat_corr(), golden_arrays(ref, net), atol=2e-5, rtol=1e-4)
+        assert_close(f"out_l{i}", on.acts[i], ref[f"out_l{i}"], atol=2e-6, stored=True)
+    assert_close("in_diff", r["in_diff"], ref["in_diff"], atol=1e-6, rtol=1e-4, stored=True)
+    assert_close("corr", on.flat_corr(), golden_arrays(ref, net), atol=2e-5, rtol=1e-4, stored=True)
     m2 = kaldi_io.read_model(d + "/out/model_out")
-    assert_close("params", on.flat_params(), m2.flat_params(), atol=1e-6)
+    assert_close("params", on.flat_params(), m2.flat_params(), atol=1e-6, stored=True)
 
 
-@pytest.mark.skipif(not oracle.have_reference("cpu"), reason="reference build (oracle/_ref) not present")
 @pytest.mark.parametrize("wl,seed", [("tiny", 1), ("small", 2), ("mid", 3)])
 def test_token_error_count_matches_reference(wl, seed):
     """Ctc::ErrorRateMSeq against the restated greedy decode + edit distance, on random-weight models whose greedy
@@ -173,7 +178,9 @@ def test_token_error_count_matches_reference(wl, seed):
         kaldi_io.write_model(d + "/model", net)
         kaldi_io.write_batch_file(d + "/batch.bin", b)
         np.save(d + "/diff.npy", np.zeros((b.feats.shape[0], w.classes), np.float32))
-        info = oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", 0.0, 0.0, diff_in=d + "/diff.npy")
+        with stored_runs(f"{wl}_token_errors", d, keep=("out/net_out.npy",), transform={"out/net_out.npy": onehot_argmax}):
+            info = oracle.run_reference("cpu", d + "/model", d + "/batch.bin", d + "/out", 0.0, 0.0,
+                                        diff_in=d + "/diff.npy")
         y = oracle.load_dump(d + "/out")["net_out"]
     err, nref = oracle.greedy_token_errors(y, b.frames, b.labels, b.S)
     assert int(info["ref_tokens"]) == nref == sum(len(l) for l in b.labels)
