@@ -14,7 +14,7 @@ OBJDIR  ?= build
 LIBDIR  ?= eesen_b200/lib
 BINDIR  := eesen_b200/bin
 
-CU_SRCS := gemm gemm_tc lstm lstm_tc ctc optim decode
+CU_SRCS := gemm gemm_tc lstm lstm_tc ctc ce optim decode
 CC_SRCS := base net abi_ops abi_net abi_decode
 CU_OBJS := $(patsubst %,$(OBJDIR)/%.cu.o,$(CU_SRCS))
 CC_OBJS := $(patsubst %,$(OBJDIR)/%.cc.o,$(CC_SRCS))

@@ -52,6 +52,7 @@ def load_library() -> C.CDLL:
     lib.eesen_b200_destroy.restype = None
     lib.eesen_b200_net_free.argtypes = [C.c_void_p]
     lib.eesen_b200_net_free.restype = None
+    lib.eesen_b200_net_last_loss.argtypes = [C.c_void_p]
     _lib = lib
     return lib
 
@@ -166,6 +167,11 @@ class Context:
     def ctc_eval(self, T, S, K, max_lab, d_len, d_labels, d_lab_len, probs, ldp, pzx, diff, ldd):
         self.check(self.lib.eesen_b200_ctc_eval(self.h, T, S, K, max_lab, _p(d_len), _p(d_labels), _p(d_lab_len),
                                                 _p(probs), ldp, _p(pzx), _p(diff), ldd), "ctc_eval")
+
+    def ce_eval(self, T, S, K, d_len, probs, ldp, d_targets, diff, ldd, d_stats):
+        """Frame-level cross-entropy (CE::EvalParallel); d_stats: device float64[3] <- obj, correct, valid frames."""
+        self.check(self.lib.eesen_b200_ce_eval(self.h, T, S, K, _p(d_len), _p(probs), ldp, _p(d_targets), _p(diff), ldd,
+                                               _p(d_stats)), "ce_eval")
 
     def sgd_update(self, w, corr, grad, n, momentum, segments: Sequence[tuple]):
         arr = (SgdSegment * len(segments))(*[SgdSegment(*s) for s in segments])
@@ -309,9 +315,43 @@ class Net:
                                                                  lab_len.ctypes.data_as(C.c_void_p), int(train)),
                        "net_train_step_device")
 
-    def read_stats(self):
+    def train_step_ce(self, feats: np.ndarray, frames: np.ndarray, targets: List[np.ndarray], train: bool = True):
+        """Frame-level cross-entropy step, HOST inputs: targets[s] holds frames[s] class ids.  Returns
+        {obj: sum of -log y[target], correct, frames: valid frames, padded: T*S rows}."""
+        feats = np.ascontiguousarray(feats, np.float32)
+        frames = np.ascontiguousarray(frames, np.int32)
+        S = frames.shape[0]
+        T = feats.shape[0] // S
+        assert all(len(t) == f for t, f in zip(targets, frames)), "one target per frame"
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(t, np.int32) for t in targets]), np.int32)
+        st = (C.c_double * 4)()
+        self.ctx.check(self.lib.eesen_b200_net_train_step_ce(self.h, feats.ctypes.data_as(C.c_void_p), T, S,
+                                                             frames.ctypes.data_as(C.c_void_p),
+                                                             flat.ctypes.data_as(C.c_void_p), int(train), st),
+                       "net_train_step_ce")
+        return self._ce_stats(st)
+
+    def train_step_ce_device(self, d_feats, T: int, S: int, frames: np.ndarray, d_targets, train: bool = True):
+        """Device-resident CE step: d_targets int32 [T*S] packed like the rows; statistics via read_stats(ce=True)."""
+        frames = np.ascontiguousarray(frames, np.int32)
+        self.ctx.check(self.lib.eesen_b200_net_train_step_ce_device(self.h, _p(d_feats), T, S,
+                                                                    frames.ctypes.data_as(C.c_void_p), _p(d_targets),
+                                                                    int(train)), "net_train_step_ce_device")
+
+    @staticmethod
+    def _ce_stats(st):
+        return {"obj": st[0], "correct": st[1], "frames": st[2], "padded": st[3]}
+
+    def read_stats(self, ce: Optional[bool] = None):
+        """Statistics of the last step, named after the loss that step used (eesen_b200_net_last_loss); passing ce
+        states the expected loss and raises if the last step used the other one."""
         st = (C.c_double * 4)()
         self.ctx.check(self.lib.eesen_b200_net_read_stats(self.h, st), "net_read_stats")
+        last_ce = bool(self.lib.eesen_b200_net_last_loss(self.h))
+        if ce is not None and bool(ce) != last_ce:
+            raise EesenB200Error(f"read_stats(ce={ce}): the last step used {'CE' if last_ce else 'CTC'}")
+        if last_ce:
+            return self._ce_stats(st)
         return {"obj": st[0], "token_err": st[1], "ref_tokens": st[2], "frames": st[3]}
 
     def get(self, which: int) -> np.ndarray:

@@ -140,6 +140,12 @@ cudaError_t ctc_eval(cudaStream_t st, int T, int S, int K, int max_lab, const in
                      const int *lab_len, const float *probs, int ldp, float *pzx, float *diff, int ldd,
                      float *ws);
 
+// ce.cu -- frame-level cross-entropy: diff = (y - onehot(target)) on rows t < len[s], 0 on the others;
+// stats[3] (device, overwritten) = sum of -log y[target], correct argmax count, valid rows
+size_t ce_workspace_bytes(int T, int S, int num_sms);
+cudaError_t ce_eval(cudaStream_t st, int num_sms, int T, int S, int K, const int *len, const float *probs, int ldp,
+                    const int *targets, float *diff, int ldd, double *stats, void *ws);
+
 // decode.cu -- one-best WFST token passing for a batch of utterances (reference src/decoder/lattice-faster-decoder.cc)
 struct DecodeGraph {      // device pointers; CSR over states, emitting arcs of a state first, then its epsilon arcs
   int num_states, num_arcs, start;

@@ -19,6 +19,8 @@ struct eesen_b200_net {
   eesen_b200_ctx *ctx;
   Net net;
   Ctc ctc;
+  CE ce;
+  bool last_ce = false;       // the loss of the last step (eesen_b200_net_read_stats)
   CuMatrix<BaseFloat> feats, net_out, obj_diff, in_diff;
   float *h_pinned = nullptr;  // pinned staging for the packed features
   size_t h_cap = 0;
@@ -28,7 +30,8 @@ struct eesen_b200_net {
   bool want_in_diff = false;
   float *d_prior = nullptr;   // log priors of the forward-only path
   size_t prior_dim = 0;
-  explicit eesen_b200_net(eesen_b200_ctx *c) : ctx(c), net(c), ctc(c) {}
+  std::vector<int32> targets;  // packed [T*S] frame targets of the host CE step
+  explicit eesen_b200_net(eesen_b200_ctx *c) : ctx(c), net(c), ctc(c), ce(c) {}
   ~eesen_b200_net() {
     if (h_pinned) cudaFreeHost(h_pinned);
     if (d_prior) cudaFree(d_prior);
@@ -55,6 +58,23 @@ static void unpack_labels(eesen_b200_net *n, int S, const int *frames, const int
   }
 }
 
+// A caller that already holds the minibatch in page-locked memory (cudaHostAlloc / cudaHostRegister) is copied from
+// directly; pageable memory goes through the pinned staging buffer first.  Either way ONE asynchronous H2D copy; the
+// steps return only after the statistics are back, so the caller's buffer is free again on return.
+static const float *stage_feats(eesen_b200_net *n, const float *feats, size_t elems) {
+  cudaPointerAttributes attr;
+  if (cudaPointerGetAttributes(&attr, feats) == cudaSuccess && attr.type == cudaMemoryTypeHost) return feats;
+  cudaGetLastError();   // a pageable pointer may leave cudaErrorInvalidValue behind on older drivers
+  if (elems > n->h_cap) {
+    if (n->h_pinned) cudaFreeHost(n->h_pinned);
+    n->h_pinned = nullptr; n->h_cap = 0;
+    if (cudaMallocHost((void **)&n->h_pinned, sizeof(float) * elems) != cudaSuccess) KALDI_ERR << "cudaMallocHost failed";
+    n->h_cap = elems;
+  }
+  memcpy(n->h_pinned, feats, sizeof(float) * elems);
+  return n->h_pinned;
+}
+
 static void run_step(eesen_b200_net *n, const CuMatrixBase<BaseFloat> &in, int train) {
   if (train) n->net.SetTrainMode(); else n->net.SetTestMode();           // train-ctc-parallel.cc:116-120
   n->net.SetSeqLengths(n->frames);                                      // train-ctc-parallel.cc:195
@@ -62,6 +82,18 @@ static void run_step(eesen_b200_net *n, const CuMatrixBase<BaseFloat> &in, int t
   n->ctc.EvalParallelAsync(n->frames, n->net_out, n->labels, &n->obj_diff);   // :199
   n->ctc.ErrorRateMSeqAsync(n->frames, n->net_out, n->labels);          // :202
   if (train) n->net.Backpropagate(n->obj_diff, n->want_in_diff ? &n->in_diff : NULL);   // :207
+  n->last_ce = false;
+}
+
+// train-ce-parallel.cc:167-177; d_targets == NULL: the host targets in n->targets (validated by CE::EvalParallel)
+static void run_step_ce(eesen_b200_net *n, const CuMatrixBase<BaseFloat> &in, const int *d_targets, int train) {
+  if (train) n->net.SetTrainMode(); else n->net.SetTestMode();
+  n->net.SetSeqLengths(n->frames);
+  n->net.Propagate(in, &n->net_out);
+  if (d_targets) n->ce.EvalParallelAsync(n->frames, n->net_out, d_targets, &n->obj_diff);
+  else n->ce.EvalParallel(n->frames, n->net_out, n->targets, &n->obj_diff);
+  if (train) n->net.Backpropagate(n->obj_diff, n->want_in_diff ? &n->in_diff : NULL);
+  n->last_ce = true;
 }
 
 extern "C" {
@@ -208,24 +240,7 @@ int eesen_b200_net_train_step(eesen_b200_net *n, const float *feats, int T, int 
     unpack_labels(n, S, frames, labels, lab_len);
     const int I = n->net.InputDim();
     size_t elems = (size_t)T * S * I;
-    // A caller that already holds the minibatch in page-locked memory (cudaHostAlloc / cudaHostRegister) is
-    // copied from directly; pageable memory goes through the pinned staging buffer first.  Either way ONE
-    // asynchronous H2D copy; the call returns only after the statistics are back, so the caller's buffer is
-    // free again on return.
-    const float *src = feats;
-    cudaPointerAttributes attr;
-    const bool pinned = cudaPointerGetAttributes(&attr, feats) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-    if (!pinned) {
-      cudaGetLastError();   // a pageable pointer may leave cudaErrorInvalidValue behind on older drivers
-      if (elems > n->h_cap) {
-        if (n->h_pinned) cudaFreeHost(n->h_pinned);
-        n->h_pinned = nullptr; n->h_cap = 0;
-        if (cudaMallocHost((void **)&n->h_pinned, sizeof(float) * elems) != cudaSuccess) KALDI_ERR << "cudaMallocHost failed";
-        n->h_cap = elems;
-      }
-      memcpy(n->h_pinned, feats, sizeof(float) * elems);
-      src = n->h_pinned;
-    }
+    const float *src = stage_feats(n, feats, elems);
     auto t1 = std::chrono::steady_clock::now();
     n->feats.Resize(T * S, I, kUndefined);
     n->feats.CopyFromHost(src, I);
@@ -264,9 +279,52 @@ int eesen_b200_net_train_step_device(eesen_b200_net *n, const float *d_feats, in
   }
 }
 
+int eesen_b200_net_train_step_ce(eesen_b200_net *n, const float *feats, int T, int S, const int *frames,
+                                 const int *targets, int train, double stats[4]) {
+  if (!n || !feats || !frames || !targets || T <= 0 || S <= 0) return EESEN_B200_EINVAL;
+  for (int s = 0; s < S; s++)
+    if (frames[s] < 0 || frames[s] > T) return n->ctx->fail(EESEN_B200_EINVAL, "frames[s] outside [0, T]");
+  try {
+    n->S = S;
+    n->frames.assign(frames, frames + S);
+    n->targets.assign((size_t)T * S, 0);
+    size_t off = 0;
+    for (int s = 0; s < S; s++)
+      for (int t = 0; t < frames[s]; t++) n->targets[(size_t)t * S + s] = targets[off++];
+    const int I = n->net.InputDim();
+    const float *src = stage_feats(n, feats, (size_t)T * S * I);
+    n->feats.Resize(T * S, I, kUndefined);
+    n->feats.CopyFromHost(src, I);
+    run_step_ce(n, n->feats, nullptr, train);
+    n->ce.Finish(stats);
+    return 0;
+  } catch (const std::exception &e) {
+    n->ctx->err = e.what();
+    return EESEN_B200_EIO;
+  }
+}
+
+int eesen_b200_net_train_step_ce_device(eesen_b200_net *n, const float *d_feats, int T, int S, const int *frames,
+                                        const int *d_targets, int train) {
+  if (!n || !d_feats || !frames || !d_targets || T <= 0 || S <= 0) return EESEN_B200_EINVAL;
+  try {
+    n->S = S;
+    n->frames.assign(frames, frames + S);
+    const int I = n->net.InputDim();
+    CuSubMatrix<BaseFloat> in(const_cast<float *>(d_feats), T * S, I, I);
+    run_step_ce(n, in, d_targets, train);
+    return 0;
+  } catch (const std::exception &e) {
+    n->ctx->err = e.what();
+    return EESEN_B200_EIO;
+  }
+}
+
+int eesen_b200_net_last_loss(const eesen_b200_net *n) { return n && n->last_ce ? 1 : 0; }
+
 int eesen_b200_net_read_stats(eesen_b200_net *n, double stats[4]) {
   if (!n || !stats) return EESEN_B200_EINVAL;
-  GUARD(n->ctx, n->ctc.Finish(stats));
+  GUARD(n->ctx, { if (n->last_ce) n->ce.Finish(stats); else n->ctc.Finish(stats); });
 }
 
 static int copy_out(const CuMatrixBase<BaseFloat> &m, float *data, int64_t cap, int *rows, int *cols) {

@@ -92,7 +92,7 @@ void eesen_b200_destroy(eesen_b200_ctx *ctx) {
   for (int i = 0; i < eesen_b200_ctx::kF16Slots; i++)
     if (ctx->f16_slots[i].planes.p) cudaFree(ctx->f16_slots[i].planes.p);
   eesen_b200_ctx::Buf *bufs[] = {&ctx->f16_meta, &ctx->f16_tmp[0], &ctx->f16_tmp[1], &ctx->f16_tmp[2], &ctx->f16_tmp[3], &ctx->decode_ws, &ctx->gemm_ws_side, &ctx->bf16_a_side, &ctx->bf16_b_side,&ctx->gemm_ws, &ctx->lstm_pbuf, &ctx->lstm_gsum, &ctx->lstm_flags,
-                                 &ctx->ctc_ws, &ctx->colsum_ws, &ctx->seg_buf, &ctx->flag_buf, &ctx->bf16_a, &ctx->bf16_b, &ctx->lstm_gflags};
+                                 &ctx->ctc_ws, &ctx->ce_ws, &ctx->colsum_ws, &ctx->seg_buf, &ctx->flag_buf, &ctx->bf16_a, &ctx->bf16_b, &ctx->lstm_gflags};
   for (auto *b : bufs)
     if (b->p) cudaFree(b->p);
   if (ctx->nccl_comm && ctx->nccl_lib) {
@@ -797,6 +797,21 @@ int eesen_b200_ctc_eval(eesen_b200_ctx *ctx, int T, int S, int K, int max_lab, c
                                (float *)ws);
   ctx->prof_end(pe);
   return ctx->check(e, "ctc_eval");
+}
+
+int eesen_b200_ce_eval(eesen_b200_ctx *ctx, int T, int S, int K, const int *d_len, const float *probs, int ldp,
+                       const int *d_targets, float *diff, int ldd, double *d_stats) {
+  if (!ctx || !d_len || !probs || !d_targets || !diff || !d_stats || T < 0 || S < 0 || K < 1 || ldp < K || ldd < K ||
+      (ldp & 3) || (ldd & 3) || (((uintptr_t)probs | (uintptr_t)diff) & 15))   // ce_kernel moves rows as float4
+    return EESEN_B200_EINVAL;
+  void *ws = nullptr;
+  int rc = ctx->reserve(ctx->ce_ws, eb::ce_workspace_bytes(T, S, ctx->num_sms), &ws);
+  if (rc) return rc;
+  ctx->launches += 2;
+  int pe = ctx->prof_begin(eesen_b200_ctx::kSoftmax);
+  cudaError_t e = eb::ce_eval(ctx->stream, ctx->num_sms, T, S, K, d_len, probs, ldp, d_targets, diff, ldd, d_stats, ws);
+  ctx->prof_end(pe);
+  return ctx->check(e, "ce_eval");
 }
 
 int eesen_b200_check_finite(eesen_b200_ctx *ctx, const float *d_x, int64_t n, int *flags) {

@@ -31,6 +31,7 @@ struct eesen_b200_ctx {
   Buf gemm_ws, lstm_pbuf, lstm_gsum, lstm_flags, ctc_ws, colsum_ws, seg_buf, flag_buf, bf16_a, bf16_b, lstm_gflags;
   Buf gemm_ws_side, bf16_a_side, bf16_b_side;   // the side stream's own scratch
   Buf decode_ws;
+  Buf ce_ws;   // per-CTA partial sums of the cross-entropy statistics
 
   // fp16x3 arithmetic (gemm_prec 0 on the 16-bit tensor pipe): converted operand planes.  Whole matrices that feed
   // several products of one layer call (d(gates), the layer input, m, Wx) are converted ONCE and registered here;

@@ -1330,4 +1330,83 @@ std::string Ctc::Report() {
   return oss.str();
 }
 
+CE::CE(eesen_b200_ctx *ctx) : ctx_(ctx) { g_ctx = ctx; }
+
+CE::~CE() {
+  if (d_len_) cudaFree(d_len_);
+  if (d_stats_) cudaFree(d_stats_);
+  if (h_stats_) cudaFreeHost(h_stats_);
+}
+
+void CE::EvalParallel(const std::vector<int32> &frame_num_utt, const CuMatrixBase<BaseFloat> &net_out,
+                      const std::vector<int32> &target, CuMatrix<BaseFloat> *diff) {
+  g_ctx = ctx_;
+  const int32 S = frame_num_utt.size(), rows = net_out.NumRows(), K = net_out.NumCols();
+  KALDI_ASSERT(S > 0 && rows % S == 0 && (int32)target.size() == rows);
+  for (int32 r = 0; r < rows; r++)   // ce-loss.cc:104-111 (the reference checks only the upper bound)
+    if (r / S < frame_num_utt[r % S] && (target[r] < 0 || target[r] >= K))
+      KALDI_ERR << "Class id out of network output dimension. Net outputs: " << K << ", class ID : " << target[r];
+  if (!pending_.empty()) Finish(NULL);   // the target buffer below is about to be overwritten
+  size_t ints = (size_t)S + rows;
+  GrowDevice(&d_len_, &cap_len_, ints);
+  CU_CHECK(cudaMemcpyAsync(d_len_ + S, target.data(), sizeof(int32) * rows, cudaMemcpyHostToDevice, Stream()));
+  EvalParallelAsync(frame_num_utt, net_out, d_len_ + S, diff);
+}
+
+void CE::EvalParallelAsync(const std::vector<int32> &frame_num_utt, const CuMatrixBase<BaseFloat> &net_out,
+                           const int32 *d_target, CuMatrix<BaseFloat> *diff) {
+  g_ctx = ctx_;
+  const int32 S = frame_num_utt.size(), rows = net_out.NumRows();
+  KALDI_ASSERT(S > 0 && rows % S == 0);
+  if ((int)pending_.size() == kSlots) Finish(NULL);
+  if (!d_stats_) {
+    CU_CHECK(cudaMalloc((void **)&d_stats_, sizeof(double) * 3 * kSlots));
+    CU_CHECK(cudaMallocHost((void **)&h_stats_, sizeof(double) * 3 * kSlots));
+  }
+  GrowDevice(&d_len_, &cap_len_, (size_t)S + (d_target == d_len_ + S ? rows : 0));
+  // pageable source: the copy is staged before cudaMemcpyAsync returns, so frame_num_utt may change afterwards
+  CU_CHECK(cudaMemcpyAsync(d_len_, frame_num_utt.data(), sizeof(int32) * S, cudaMemcpyHostToDevice, Stream()));
+  diff->Resize(rows, net_out.NumCols(), kUndefined);
+  CheckAbi(ctx_, eesen_b200_ce_eval(ctx_, rows / S, S, net_out.NumCols(), d_len_, net_out.Data(), net_out.Stride(),
+                                    d_target, diff->Data(), diff->Stride(), d_stats_ + 3 * pending_.size()),
+           "eesen_b200_ce_eval");
+  pending_.push_back(Pending{S, rows});
+}
+
+void CE::Finish(double stats[4]) {
+  if (!pending_.empty()) {
+    const size_t n = pending_.size();
+    CU_CHECK(cudaMemcpyAsync(h_stats_, d_stats_, sizeof(double) * 3 * n, cudaMemcpyDeviceToHost, Stream()));
+    CU_CHECK(SyncStream());
+    for (size_t i = 0; i < n; i++) {
+      const double obj = h_stats_[3 * i], correct = h_stats_[3 * i + 1], valid = h_stats_[3 * i + 2];
+      const int64 S = pending_[i].S, rows = pending_[i].rows;
+      obj_ += obj; obj_progress_ += obj;                              // ce-loss.cc:144-150
+      correct_ += (int64)correct; correct_progress_ += (int64)correct;
+      sequences_progress_ += S; sequences_num_ += S;
+      frames_progress_ += rows; frames_ += rows;                      // padded rows, as the reference counts them
+      if (sequences_progress_ > report_step_) {                       // ce-loss.cc:152-167
+        KALDI_LOG << "After " << sequences_num_ << " sequences (" << frames_ / (100.0 * 3600) << "Hr): "
+                  << "CE-Obj = " << obj_progress_ / sequences_progress_
+                  << "Frame-level CE-Obj = " << obj_progress_ / frames_progress_
+                  << "   FrameAcc = " << 100.0 * (double(correct_progress_) / frames_progress_) << "%"
+                  << " obj_progress_=  " << obj_progress_
+                  << " sequences_progress_=  " << sequences_progress_
+                  << " frames_progress_=  " << frames_progress_;
+        sequences_progress_ = 0; frames_progress_ = 0; obj_progress_ = 0.0; correct_progress_ = 0;
+      }
+      last_[0] = obj; last_[1] = correct; last_[2] = valid; last_[3] = (double)rows;
+    }
+    pending_.clear();
+  }
+  if (stats) memcpy(stats, last_, sizeof(last_));
+}
+
+std::string CE::Report() {
+  Finish(NULL);
+  std::ostringstream oss;
+  oss << "\nFRAME_ACCURACY >> " << 100.0 * (double(correct_) / frames_) << "% <<";   // ce-loss.cc:171-175, real quotient
+  return oss.str();
+}
+
 }  // namespace eesen

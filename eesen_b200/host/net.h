@@ -408,5 +408,42 @@ class Ctc {
   int32 max_lab_ = 1;
 };
 
+// ce-loss.h:32-86, the parallel half.  The rows valid in the mask are t < frame_num_utt[s] (no float mask); the
+// statistics of each call stay on the device and are folded, in call order, at the next Finish() -- with the
+// reference's progress lines -- so that a training loop never waits for the device per minibatch.
+// Deliberate differences (DESIGN.md section 5): 64-bit counters, Report() prints the real quotient, the
+// objective reads the target column only.
+class CE {
+ public:
+  explicit CE(eesen_b200_ctx *ctx);
+  ~CE();
+  // target: [T*S] packed like the rows of net_out; entries of padded rows are ignored, the others must lie in [0, K)
+  void EvalParallel(const std::vector<int32> &frame_num_utt, const CuMatrixBase<BaseFloat> &net_out,
+                    const std::vector<int32> &target, CuMatrix<BaseFloat> *diff);
+  // the same with the packed targets already on the device (validated by the caller)
+  void EvalParallelAsync(const std::vector<int32> &frame_num_utt, const CuMatrixBase<BaseFloat> &net_out,
+                         const int32 *d_target, CuMatrix<BaseFloat> *diff);
+  void SetReportStep(int32 report_step) { report_step_ = report_step; }
+  std::string Report();
+  // waits, folds every pending call; stats (may be NULL) of the last call: obj, correct, valid frames, padded rows
+  void Finish(double stats[4]);
+
+ private:
+  eesen_b200_ctx *ctx_;
+  int64 frames_ = 0, sequences_num_ = 0, correct_ = 0;
+  double obj_ = 0;
+  int64 frames_progress_ = 0, sequences_progress_ = 0, correct_progress_ = 0;
+  double obj_progress_ = 0;
+  int32 report_step_ = 100;
+  int *d_len_ = nullptr;         // [S] lengths, then [T*S] targets (host-target calls)
+  size_t cap_len_ = 0;
+  double *d_stats_ = nullptr;    // [kSlots][3] one slot per pending call
+  double *h_stats_ = nullptr;    // pinned mirror
+  static const int kSlots = 64;
+  struct Pending { int32 S, rows; };
+  std::vector<Pending> pending_;
+  double last_[4] = {0, 0, 0, 0};
+};
+
 }  // namespace eesen
 #endif

@@ -190,6 +190,20 @@ int eesen_b200_ctc_eval(eesen_b200_ctx *ctx, int T, int S, int K, int max_lab, c
                         const int *d_labels, const int *d_lab_len, const float *probs, int ldp,
                         float *pzx, float *diff, int ldd);
 
+/* CE::EvalParallel compute (reference src/net/ce-loss.cc:94-169), frame-level cross-entropy.
+ *   probs     [T*S x K] (ldp) softmax outputs           d_len[S] valid frames: row t*S+s is valid iff t < d_len[s]
+ *   ldp, ldd must be multiples of 4 and probs, diff 16-byte aligned (rows are moved as float4): EESEN_B200_EINVAL
+ *   otherwise
+ *   d_targets [T*S] int32, packed like the rows; the class of each valid row, in [0, K) (padded rows ignored)
+ *   diff      [T*S x K] (ldd) out: y - onehot(target) on valid rows (d(CE)/d(logits)), exactly 0 on padded rows;
+ *             columns [K, ldd) untouched
+ *   d_stats   double[3] (device), overwritten: [0] sum over valid rows of -log y[target] (the target column only,
+ *             so a posterior of 0 elsewhere leaves it finite), [1] valid rows whose first row maximum is the
+ *             target (FindRowMaxId tie rule), [2] valid rows.  A valid row with a target outside [0, K) makes [0]
+ *             NaN; nothing outside the row is read.  The statistics are the same bits on every run. */
+int eesen_b200_ce_eval(eesen_b200_ctx *ctx, int T, int S, int K, const int *d_len, const float *probs, int ldp,
+                       const int *d_targets, float *diff, int ldd, double *d_stats);
+
 /* Momentum + clip + SGD over a contiguous arena (reference src/net/bilstm-layer.h:846-883,
  * affine-trans-layer.h:182-195):  corr = grad + momentum*corr; clamp(corr, +-max_grad); w -= lr*corr.
  * segments (host memory) partition [0, n): lr = learn_rate*learn_rate_coef, max_grad <= 0 disables clipping. */
@@ -255,7 +269,24 @@ int eesen_b200_net_train_step(eesen_b200_net *net, const float *feats, int T, in
  * statistics stay on the device until eesen_b200_net_read_stats. */
 int eesen_b200_net_train_step_device(eesen_b200_net *net, const float *d_feats, int T, int S,
                                      const int *frames, const int *labels, const int *lab_len, int train);
+/* The same step with frame-level cross-entropy instead of CTC (reference src/netbin/train-ce-parallel.cc:167-177):
+ * SetSeqLengths, Propagate, CE::EvalParallel and -- if train != 0 -- Backpropagate with the all-reduce and the
+ * update.  HOST inputs; blocks until the statistics are back.
+ *   feats [T*S x I] packed, frames[S], targets: concatenated per utterance, frames[s] class ids each, in [0, K)
+ *   stats out: [0] sum of -log y[target] over valid frames  [1] correctly classified frames  [2] valid frames
+ *              [3] padded rows (T*S, the reference's frame count) */
+int eesen_b200_net_train_step_ce(eesen_b200_net *net, const float *feats, int T, int S, const int *frames,
+                                 const int *targets, int train, double stats[4]);
+/* Same step with inputs ALREADY RESIDENT on the device: d_feats [T*S x I] (ld = I), d_targets [T*S] packed like the
+ * rows (padded rows ignored, the caller guarantees [0, K)); frames[S] on the host.  Asynchronous: statistics stay on
+ * the device until eesen_b200_net_read_stats.  Targets are NOT checked here: a valid row with a target outside [0, K)
+ * gets no -1 in its gradient and makes stats[0] NaN, so a caller that has not validated its targets checks that. */
+int eesen_b200_net_train_step_ce_device(eesen_b200_net *net, const float *d_feats, int T, int S, const int *frames,
+                                        const int *d_targets, int train);
+/* Statistics of the last step, whichever loss it used (layouts above). */
 int eesen_b200_net_read_stats(eesen_b200_net *net, double stats[4]);
+/* The loss of the last step: 0 = CTC (or no step yet), 1 = frame-level cross-entropy. */
+int eesen_b200_net_last_loss(const eesen_b200_net *net);
 
 /* ---------------------------------------------------------------- forward-only path (SURVEY.md 8f N2)
  * One packed batch through what reference src/netbin/net-output-extract.cc:83-118 does per
@@ -279,7 +310,7 @@ int eesen_b200_net_write_nonparallel(eesen_b200_net *net, const char *path, int 
 
 /* Introspection for the parity tests (host copies, synchronous).  which:
  *   0..L    Net::propagate_buf_[which]     (layer inputs/outputs, L = num_layers)
- *   100     obj_diff (CTC gradient wrt logits)      101  per-utterance pzx [S]
+ *   100     obj_diff (CTC or CE gradient wrt logits, from the last step)      101  per-utterance pzx [S]
  *   102     in_diff  (gradient wrt the network input)
  *   200     parameters   201 momentum buffers (corr)   202 raw gradients of the last step (after all-reduce)
  *   203     Adagrad/RMSProp accumulators (zeros while none exist)
