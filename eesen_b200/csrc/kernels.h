@@ -69,7 +69,6 @@ struct LstmFwdArgs {
   const unsigned *gflag = nullptr;
   unsigned gepoch = 0;
   int gchunk = 0, gready = 0;
-  int tune = 0;   // debug knobs (EESEN_B200_TUNE): bit 0 = first exchange poll behind the saved-state stores
   // (tcgen05 engine) fp16 planes of the layer output for the dense products that read it next (the input product of the
   // layer above, the weight gradients): hi = fp16(2^13 * m), lo = fp16(2^13 * m - hi) -- |m| < 1, so the scale is fixed
   // and the kernel can write them next to m itself; [T*S x ldh] halfs each, dir d at col d*C.  NULL: not wanted.
@@ -90,13 +89,6 @@ struct LstmBwdArgs {
   int drop = 0;                 // as LstmFwdArgs (:604-879)
   const float *rmask = nullptr;
   int ldr = 0, rmask_per_step = 0;
-  int tune = 0;                 // debug knobs (EESEN_B200_TUNE): bit 1 = 64-row remainder tile from shared memory (SS form)
-  // Streamed dout (tcgen05 engine): dout arrives in PAIRS of time chunks of `dchunk` positions, pair ci = chunk ci from
-  // the start and chunk ci from the end of the sequence (dnck chunks in all); pair ci may be read once dflag[ci] ==
-  // depoch, pairs < dready were complete before the launch.  dflag == nullptr: everything is there.
-  const unsigned *dflag = nullptr;
-  unsigned depoch = 0;
-  int dchunk = 0, dnck = 0, dready = 0;
   unsigned *dgmax = nullptr;    // (tcgen05 engine) atomicMax of the bits of max |DG| over the launch, or NULL
 };
 struct LstmPlan {

@@ -203,15 +203,14 @@ __device__ __forceinline__ void issue_bwd_tile_stacked(uint32_t tA, uint64_t dB,
     umma_f16_ts(tmem, tA + ks * 8, dB + (uint64_t)((kb * 4096 + k4 * 32) >> 4), idN, ks != 0);
   }
 }
-template <int ROWS>
 __device__ __forceinline__ void issue_bwd_tile(uint64_t dAhi, uint64_t dAlo, uint64_t dB, uint32_t tmem) {
-  const uint32_t idN = idesc_f16(ROWS, 32), idH = idesc_f16(ROWS, 16);
+  const uint32_t idN = idesc_f16(128, 32), idH = idesc_f16(128, 16);
 #pragma unroll
   for (int ks = 0; ks < 8; ks++) {
     const int kb = ks >> 2, k4 = ks & 3;
     const uint64_t bd = dB + (uint64_t)((kb * 4096 + k4 * 32) >> 4);
-    umma_f16(tmem, dAhi + (uint64_t)((kb * ROWS * 128 + k4 * 32) >> 4), bd, idN, ks != 0);
-    umma_f16(tmem + 32, dAlo + (uint64_t)((kb * ROWS * 128 + k4 * 32) >> 4), bd, idH, ks != 0);
+    umma_f16(tmem, dAhi + (uint64_t)((kb * 16384 + k4 * 32) >> 4), bd, idN, ks != 0);
+    umma_f16(tmem + 32, dAlo + (uint64_t)((kb * 16384 + k4 * 32) >> 4), bd, idH, ks != 0);
   }
 }
 
@@ -564,7 +563,7 @@ lstm_tc_fwd_kernel(LstmFwdArgs a, int groups, int ndir) {
           if (step + 1 < T) {
             uint32_t h, l;
             split_f16(sm[e], h, l);
-            st_word(xbuf + (((size_t)((step & 1) * ndir + dir) * groups + group) * TCL_UG + 2 * up + e) * C + cell,
+            st_word(xbuf + (((size_t)((step & 1) * ndir + dir) * groups + group) * TCL_UG) * C + (size_t)(2 * up + e) * C + cell,
                     h | ((l & 0xfffeu) << 16) | ((uint32_t)((step >> 1) & 1) << 16));   // tag = LSB of lo'
           }
           __stcs(a.out + ((size_t)t * S + uidx[e]) * a.ldo + (size_t)dir * C + cell, sm[e]);
@@ -578,7 +577,7 @@ lstm_tc_fwd_kernel(LstmFwdArgs a, int groups, int ndir) {
         for (int i = 0; i < MAXT; i++)
           if (live[i]) { xq[i][0] = ld_word4(xn + xoff[i]); xq[i][1] = ld_word4(xn + xoff[i] + 1); }
       };
-      if (!CL && step + 1 < T && !(a.tune & 1)) first_poll();
+      if (!CL && step + 1 < T) first_poll();
       TC_TICK(0, 3);
 #pragma unroll
       for (int e = 0; e < 2; e++) {
@@ -589,7 +588,6 @@ lstm_tc_fwd_kernel(LstmFwdArgs a, int groups, int ndir) {
           __stcs(a.cell + ((size_t)t * S + uidx[e]) * a.ldc + (size_t)dir * C + cell, sc[e]);
         }
       }
-      if (!CL && step + 1 < T && (a.tune & 1)) first_poll();
       if (step + 1 < T) {
         if (a.gflag) {   // streamed input product: the next position may lie in a chunk that is still being computed
           const int need = (step + 1) / a.gchunk;
@@ -630,8 +628,6 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
   uint8_t *smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   const int C = a.C, S = a.S, T = a.T;
   const int n128 = C >> 7, rem64 = (C & 127) ? 1 : 0, MT = n128 + rem64;
-  const bool ss64 = !CL && rem64 && (a.tune & 2);         // debug: the 64-row tile as an M = 64 SS-form tile, issued last
-  const bool stk = rem64 && !ss64;                        // default: stacked TMEM tile, issued first
   const int NTS = n128 < 2 ? n128 : 2;                    // full tiles resident in TMEM
   uint8_t *Bt = smem;                                     // [2 k-blocks][32 rows][128 B]
   // [2 step parities][16] inverse column scales.  Two sets: a warp may write the scales of step s+1 while another warp of
@@ -645,10 +641,10 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
   float *red = ysm + TCL_UG * 64;                         // [7][16 utts][32 cells] bias / peephole sums at the end
   uint8_t *Ahi = smem + 32768;                            // full tiles beyond the TMEM-resident ones: [2 k-blocks][128][128 B] each
   uint8_t *Alo = Ahi + (size_t)(n128 - NTS) * 32768;
-  uint8_t *Ahi64 = Alo + (size_t)(n128 - NTS) * 32768;    // (ss64 only) [2 k-blocks][64 rows][128 B], hi then lo'
-  uint8_t *Alo64 = Ahi64 + 16384;
   constexpr int kRRow = 20, kRBlk = 32 * kRRow;           // (CL) floats per cell row (16 utts + pad: 80 B) / per producer block
-  float *R = reinterpret_cast<float *>(Alo64 + 16384);    // (CL) [2 parity][slices][32 cells][kRRow]
+  // (CL) [2 parity][slices][32 cells][kRRow], behind 32 KB of unused padding: kept so that tc_bwd_smem, and with it which
+  // plans fit (occupancy, cluster eligibility), stays as measured
+  float *R = reinterpret_cast<float *>(Alo + (size_t)(n128 - NTS) * 32768 + 32768);
   const uint32_t rbytes = (uint32_t)slices * 2048u;       // (CL) payload bytes a CTA receives per step
   __shared__ uint64_t b_full, mma_done[4], rfull[2];   // one commit barrier per M tile (at most 4 tiles)
   __shared__ uint32_t tmem_base_sm;
@@ -679,16 +675,6 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
         *reinterpret_cast<uint16_t *>(Ahi + off) = (uint16_t)h;
         *reinterpret_cast<uint16_t *>(Alo + off) = (uint16_t)l;
       }
-    }
-  }
-  if (ss64) {
-    for (int idx = tid; idx < 128 * 64; idx += TCL_THREADS) {
-      const int kk = idx >> 6, r = idx & 63;
-      const float w = __ldg(P.wm + ((size_t)(kk >> 5) * C + slice * TCL_CS + (kk & 31)) * P.ldwm + n128 * 128 + r);
-      uint32_t h, l;
-      split_f16(w, h, l);
-      *reinterpret_cast<uint16_t *>(Ahi64 + sw128_off(64, r, kk)) = (uint16_t)h;
-      *reinterpret_cast<uint16_t *>(Alo64 + sw128_off(64, r, kk)) = (uint16_t)l;
     }
   }
   for (int idx = tid; idx < 2048; idx += TCL_THREADS) reinterpret_cast<uint32_t *>(Bt)[idx] = 0u;
@@ -745,7 +731,7 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
   }
   // the stacked tile of the last 64 rows (columns [160 + 128 * NTS, + 64)): lane quadrants 0-1 hold hi, 2-3 lo'
   const uint32_t colS = kColA + (uint32_t)NTS * 128;
-  if (stk) {
+  if (rem64) {
     const int j = n128 * 128 + (warp & 1) * 32 + lane;
     const bool lo_half = (warp & 2) != 0;
     const uint32_t tl = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + colS;
@@ -792,12 +778,7 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
     float vg[2], vi[2], vf[2], vo[2], vc[2], vcp[2], vd[2], vr[2] = {1.f, 1.f};
     float runmax = 0.f;
     const int tstep = dir == 0 ? -1 : 1;   // time order of the forward pass: c_prev lives at t + tstep
-    int dhave = a.dready - 1;                              // last pair of dout chunks known to be complete
     auto prefetch = [&](int t) {
-      if (a.dflag) {   // streamed dX of the layer above: position t may lie in a pair of chunks still being computed
-        const int k = t / a.dchunk, need = min(k, a.dnck - 1 - k);
-        if (need > dhave) { wait_flag(a.dflag + need, a.depoch); dhave = need; }
-      }
 #pragma unroll
       for (int e = 0; e < 2; e++) {
         if (!ok[e]) { vg[e] = vi[e] = vf[e] = vo[e] = vc[e] = vcp[e] = vd[e] = 0.f; continue; }
@@ -945,18 +926,14 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
           // one commit per M tile: the epilogue (TMEM -> partial words) of a tile runs while the tensor pipe is
           // still working on the next one.  The stacked tile goes first: its epilogue has one more hand-over.
           int nb = 0;
-          if (stk) {
+          if (rem64) {
             issue_bwd_tile_stacked(tmem_base + colS, dBt, tmem_base + accS);
             umma_commit(&mma_done[nb++]);
           }
           for (int mt = 0; mt < n128; mt++) {
             const uint64_t toff = (uint64_t)(((mt - NTS) * 32768) >> 4);
             if (mt < NTS) issue_bwd_tile_ts(tmem_base + kColA + mt * 128, tmem_base + kColA + mt * 128 + 64, dBt, tmem_base + acc_col(mt));
-            else issue_bwd_tile<128>(dAhi + toff, dAlo + toff, dBt, tmem_base + acc_col(mt));
-            umma_commit(&mma_done[nb++]);
-          }
-          if (ss64) {
-            issue_bwd_tile<64>(umma_desc(smem_u32(Ahi64), 16, 1024, 2), umma_desc(smem_u32(Alo64), 16, 1024, 2), dBt, tmem_base + accS);
+            else issue_bwd_tile(dAhi + toff, dAlo + toff, dBt, tmem_base + acc_col(mt));
             umma_commit(&mma_done[nb++]);
           }
         }
@@ -977,11 +954,10 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
         // Warp 0 issues the MMAs and is the last to get to the epilogue; every consumer of the cluster waits for ITS
         // pushes (ncu stall samples, profiles/r02_p_lstm_tc_hotspots.txt: 27 % of all warp time in the wait for the peers'
         // partials).  So warp 0 takes no part in the epilogue: warp 4, which owns the same TMEM lane quadrant, handles
-        // both utterance halves while warp 0 is still issuing.  (EESEN_B200_TUNE bit 6: the old split, A/B.)
-        const bool relieve = !(a.tune & 64);
-        const bool w0 = relieve && warp == 0;
-        const int nhalves = (relieve && warp == 4) ? 2 : 1;
-        const int nbar2 = relieve ? 224 : 256;   // threads on the stacked tile's hand-over barrier
+        // both utterance halves while warp 0 is still issuing (profiles/r02_v_ab.txt).
+        const bool w0 = warp == 0;
+        const int nhalves = warp == 4 ? 2 : 1;
+        const int nbar2 = 224;   // threads on the stacked tile's hand-over barrier
         // (CL) the 8 utterance values of accumulator row `row` of the 32-row block that belongs to CTA d of the cluster:
         // two 16-byte stores into d's receive buffer (step & 1), block `slice` (= this producer), complete_tx on d's barrier
         auto push8 = [&](uint32_t d, int row, int uhh, const float (&pv)[8]) {
@@ -1003,7 +979,7 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
           if (w0) continue;
           // (the column scales were written by the other warps before they arrived on b_full: they are read only behind a
           // commit, which is behind b_full; two sets by step parity, see the declaration of scl)
-          if (stk && bi == 0) {
+          if (rem64 && bi == 0) {
             // stacked tile: lanes 0-63 (quadrants 0-1) carry hi*hi | hi*lo', lanes 64-127 the lo'*hi term of the same
             // rows -- it crosses to the other warps through shared memory
             const uint32_t tl = tmem_base + ((uint32_t)(quad * 32) << 16) + accS;
@@ -1043,8 +1019,7 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
             TC_TICK(1, 3);
             continue;
           }
-          const int mt = bi - (stk ? 1 : 0);
-          const bool full = mt < n128;              // (ss64: the last one is the M = 64 tile)
+          const int mt = bi - rem64;
           const uint32_t tl = tmem_base + ((uint32_t)(quad * 32) << 16) + acc_col(mt);
           for (int hh = 0; hh < nhalves; hh++) {
             const int uhh = nhalves == 2 ? 1 - hh : uh;
@@ -1054,22 +1029,19 @@ lstm_tc_bwd_kernel(LstmBwdArgs a, int groups, int slices, int ndir) {
             tmem_ld8(tl + 32 + 8 * uhh, y0);
             tmem_ld_wait();
             TC_OBS(1);
-            // M = 128: lane = row; M = 64: rows 16*quad .. +15 sit in lanes 0-15 of every quadrant
-            const int j = full ? mt * 128 + quad * 32 + lane : mt * 128 + quad * 16 + lane;
-            if (full || lane < 16) {
-              float pv[8];
+            const int j = mt * 128 + quad * 32 + lane;   // lane = row
+            float pv[8];
+#pragma unroll
+            for (int jj = 0; jj < 8; jj++)
+              pv[jj] = (u2f(x0[jj]) + (u2f(x1[jj]) + u2f(y0[jj])) * kLoUnscale) * scl[(step & 1) * 16 + 8 * uhh + jj];
+            TC_OBS(2);
+            if (CL) {
+              push8((uint32_t)(mt * 4 + quad), lane, uhh, pv);
+              TC_OBS(3);
+            } else {
 #pragma unroll
               for (int jj = 0; jj < 8; jj++)
-                pv[jj] = (u2f(x0[jj]) + (u2f(x1[jj]) + u2f(y0[jj])) * kLoUnscale) * scl[(step & 1) * 16 + 8 * uhh + jj];
-              TC_OBS(2);
-              if (CL) {
-                push8((uint32_t)(mt * 4 + quad), lane, uhh, pv);   // (CL: full tiles only)
-                TC_OBS(3);
-              } else {
-#pragma unroll
-                for (int jj = 0; jj < 8; jj++)
-                  st_word(pw + (size_t)(8 * uhh + jj) * C + j, (__float_as_uint(pv[jj]) & 0xfffffffeu) | tagw);   // tag = LSB
-              }
+                st_word(pw + (size_t)(8 * uhh + jj) * C + j, (__float_as_uint(pv[jj]) & 0xfffffffeu) | tagw);   // tag = LSB
             }
           }
           TC_TICK(1, 3);
@@ -1129,7 +1101,7 @@ size_t tc_fwd_smem(int C) {
 // like the forward kernel it asks for most of the SM so that no TMEM-allocating GEMM CTA lands beside it
 size_t tc_bwd_smem(int C) {
   const int n128 = C >> 7, nts = n128 < 2 ? n128 : 2;
-  const size_t need = 32768 + (size_t)(n128 - nts) * 65536 + 32768 + 1024 +   // (+ 32 KB: the debug SS form of the 64-row tile)
+  const size_t need = 32768 + (size_t)(n128 - nts) * 65536 + 32768 + 1024 +   // (+ 32 KB unused, see lstm_tc_bwd_kernel)
                       (C <= 384 ? (size_t)2 * (C / TCL_CS) * 32 * 80 : 0);
   return need > 180 * 1024 ? need : (size_t)180 * 1024;
 }

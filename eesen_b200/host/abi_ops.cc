@@ -18,6 +18,17 @@ static std::string g_create_error;
     if (rc__) return rc__;                    \
   } while (0)
 
+// n kernels launched by f() on the stream of on_side, timed under profile category cat (kUntimed: not timed)
+enum { kUntimed = -1 };
+template <class F>
+static int launch(eesen_b200_ctx *ctx, int cat, int n, const char *what, F &&f, bool on_side = false) {
+  ctx->launches += n;
+  const int pe = cat == kUntimed ? -1 : ctx->prof_begin(cat, on_side);
+  const cudaError_t e = f();
+  ctx->prof_end(pe);
+  return ctx->check(e, what);
+}
+
 extern "C" {
 
 int eesen_b200_create(eesen_b200_ctx **out, int device) {
@@ -59,16 +70,6 @@ int eesen_b200_create(eesen_b200_ctx **out, int device) {
   {
     const char *ov = getenv("EESEN_B200_OVERLAP");
     ctx->overlap = (ov && ov[0] == '0') ? 0 : 1;
-    const char *sg = getenv("EESEN_B200_STREAM_GEMM");
-    ctx->stream_gemm = (sg && sg[0] == '0') ? 0 : 1;
-    const char *sx = getenv("EESEN_B200_STREAM_DX");
-    ctx->stream_dx = (sx && sx[0] == '1') ? 1 : 0;
-    const char *dr = getenv("EESEN_B200_DX_READY");
-    ctx->dx_ready_pairs = dr ? std::max(1, atoi(dr)) : 1;
-    const char *fr = getenv("EESEN_B200_FWD_READY");
-    ctx->fwd_ready_chunks = fr ? std::max(1, atoi(fr)) : 1;
-    const char *ec = getenv("EESEN_B200_EARLY_CONV");
-    ctx->early_conv = (ec && ec[0] == '0') ? 0 : 1;
     const char *fx = getenv("EESEN_B200_GEMM_FP32X3");
     ctx->f16x3 = (fx && std::string(fx) == "tf32") ? 0 : 1;
   }
@@ -89,8 +90,10 @@ void eesen_b200_destroy(eesen_b200_ctx *ctx) {
   cudaSetDevice(ctx->device);
   ctx->join_side();
   cudaStreamSynchronize(ctx->stream);
-  for (int i = 0; i < eesen_b200_ctx::kF16Slots; i++)
-    if (ctx->f16_slots[i].planes.p) cudaFree(ctx->f16_slots[i].planes.p);
+  for (const auto &e : ctx->f16_slots)
+    if (e.planes.p) cudaFree(e.planes.p);
+  for (const auto &e : ctx->act)
+    if (e.planes.p) cudaFree(e.planes.p);
   eesen_b200_ctx::Buf *bufs[] = {&ctx->f16_meta, &ctx->f16_tmp[0], &ctx->f16_tmp[1], &ctx->f16_tmp[2], &ctx->f16_tmp[3], &ctx->decode_ws, &ctx->gemm_ws_side, &ctx->bf16_a_side, &ctx->bf16_b_side,&ctx->gemm_ws, &ctx->lstm_pbuf, &ctx->lstm_gsum, &ctx->lstm_flags,
                                  &ctx->ctc_ws, &ctx->ce_ws, &ctx->colsum_ws, &ctx->seg_buf, &ctx->flag_buf, &ctx->bf16_a, &ctx->bf16_b, &ctx->lstm_gflags};
   for (auto *b : bufs)
@@ -129,6 +132,7 @@ int eesen_b200_sm_count(const eesen_b200_ctx *ctx) { return ctx->num_sms; }
 long eesen_b200_launch_count(const eesen_b200_ctx *ctx) { return ctx->launches; }
 
 // ---- fp16x3 operand planes --------------------------------------------------------------------------------------
+// record idx of f16_meta (eesen_b200_ctx::kMeta*): {max scratch, kexp}
 static int f16_meta(eesen_b200_ctx *ctx, int idx, unsigned **mx, int **kexp) {
   void *m = nullptr;
   int rc = ctx->reserve(ctx->f16_meta, 4096, &m);
@@ -138,216 +142,162 @@ static int f16_meta(eesen_b200_ctx *ctx, int idx, unsigned **mx, int **kexp) {
   return 0;
 }
 
-static bool f16_lookup(eesen_b200_ctx *ctx, const float *P, long r, int c, int ld, eb::F16View *out);
-
-// convert the whole matrix [rows x cols] (ld) on `stream` and remember it: later products find sub-blocks by address
-// persist (only while a Net drives a training forward pass, ctx->act_enable): the planes go to an ActPlanes slot and stay
-// valid until the next forward pass -- the input weights Wx, which the dX product of the backward pass reads again
-static int f16_register(eesen_b200_ctx *ctx, const float *base, long rows, int cols, int ld, bool on_side = false,
-                        const unsigned *known_max = nullptr, bool persist = false) {
-  if (!ctx->f16x3 || ctx->gemm_prec != 0 || ctx->gemm_engine != 0 || !base || rows <= 0 || cols <= 0) return 0;
-  { eb::F16View have; if (f16_lookup(ctx, base, rows, cols, ld, &have)) return 0; }   // (e.g. planes the forward kernel wrote)
-  if (persist && ctx->act_enable) {
-    int slot = -1;
-    for (int i = 0; i < eesen_b200_ctx::kActSlots; i++)
-      if (ctx->act[i].base == base) slot = i;
-    if (slot < 0) { slot = ctx->act_next; ctx->act_next = (ctx->act_next + 1) % eesen_b200_ctx::kActSlots; }
-    eesen_b200_ctx::ActPlanes &e = ctx->act[slot];
-    const size_t pb = eb::f16x2_plane_bytes(rows, cols);
-    void *pl = nullptr;
-    int rc = ctx->reserve(e.planes, 2 * pb + 256, &pl);
-    if (rc) return rc;
-    unsigned *mx; int *kx;
-    if ((rc = f16_meta(ctx, eesen_b200_ctx::kF16Slots + 8 + slot, &mx, &kx))) return rc;
-    e.base = base; e.rows = rows; e.cols = cols; e.ld = ld; e.ldd = (cols + 7) & ~7; e.gen = ctx->act_gen;
-    e.view.hi = pl; e.view.lo = (char *)pl + ((pb + 255) & ~(size_t)255); e.view.ld = e.ldd; e.view.kexp = kx;
-    int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-    cudaError_t ce = eb::convert_f16x2(on_side ? ctx->side : ctx->stream, ctx->num_sms, base, rows, cols, ld, (void *)e.view.hi,
-                                       (void *)e.view.lo, mx, kx, known_max);
-    ctx->prof_end(pe);
-    ctx->launches += known_max ? 1 : 2;
-    return ctx->check(ce, "convert_f16x2");
-  }
-  if (ctx->f16_used >= eesen_b200_ctx::kF16Slots) return 0;   // (falls back to per-call conversion)
-  eesen_b200_ctx::F16Entry &e = ctx->f16_slots[ctx->f16_used];
+// hi / lo planes [rows x ldd] in `planes`, both 256-byte aligned
+static int reserve_planes(eesen_b200_ctx *ctx, eesen_b200_ctx::Buf &planes, long rows, int cols, int ldd, eb::F16View *view) {
   const size_t pb = eb::f16x2_plane_bytes(rows, cols);
   void *pl = nullptr;
-  int rc = ctx->reserve(e.planes, 2 * pb + 256, &pl);
+  int rc = ctx->reserve(planes, 2 * pb + 256, &pl);
   if (rc) return rc;
-  unsigned *mx; int *kx;
-  if ((rc = f16_meta(ctx, ctx->f16_used, &mx, &kx))) return rc;
-  e.base = base; e.rows = rows; e.cols = cols; e.ld = ld; e.ldd = (cols + 7) & ~7;
-  e.view.hi = pl; e.view.lo = (char *)pl + ((pb + 255) & ~(size_t)255); e.view.ld = e.ldd; e.view.kexp = kx;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-  cudaError_t ce = eb::convert_f16x2(on_side ? ctx->side : ctx->stream, ctx->num_sms, base, rows, cols, ld, (void *)e.view.hi,
-                                     (void *)e.view.lo, mx, kx, known_max);
-  ctx->prof_end(pe);
-  ctx->launches += known_max ? 1 : 2;
-  if ((rc = ctx->check(ce, "convert_f16x2"))) return rc;
-  ctx->f16_used++;
+  view->hi = pl; view->lo = (char *)pl + ((pb + 255) & ~(size_t)255); view->ld = ldd;
   return 0;
+}
+
+// convert src [rows x cols] (ld) into planes on the stream of on_side; the scan scratch and the scale exponent go to
+// f16_meta record `meta`.  timed: as a product of that stream (else it is timed inside the product it feeds).
+static int convert_planes(eesen_b200_ctx *ctx, eesen_b200_ctx::Buf &planes, int meta, const float *src, long rows, int cols,
+                          int ld, bool on_side, const unsigned *known_max, bool timed, eb::F16View *view) {
+  unsigned *mx; int *kx;
+  int rc;
+  if ((rc = reserve_planes(ctx, planes, rows, cols, (cols + 7) & ~7, view))) return rc;
+  if ((rc = f16_meta(ctx, meta, &mx, &kx))) return rc;
+  view->kexp = kx;
+  return launch(ctx, timed ? (int)eesen_b200_ctx::kGemm : kUntimed, known_max ? 1 : 2, "convert_f16x2", [&] {
+    return eb::convert_f16x2(on_side ? ctx->side : ctx->stream, ctx->num_sms, src, rows, cols, ld, (void *)view->hi,
+                             (void *)view->lo, mx, kx, known_max);
+  }, on_side);
+}
+
+// the per-pass entry of `base`: its own slot, else the next one round robin
+static int act_slot(eesen_b200_ctx *ctx, const float *base) {
+  int slot = -1;
+  for (int i = 0; i < eesen_b200_ctx::kActSlots; i++)
+    if (ctx->act[i].base == base) slot = i;
+  if (slot < 0) { slot = ctx->act_next; ctx->act_next = (ctx->act_next + 1) % eesen_b200_ctx::kActSlots; }
+  return slot;
 }
 
 // a [r x c] block at P with leading dimension ld: inside a registered matrix (or a layer output whose planes the
 // recurrent forward kernel wrote during this forward pass)?
 static bool f16_lookup(eesen_b200_ctx *ctx, const float *P, long r, int c, int ld, eb::F16View *out) {
-  for (int i = 0; i < ctx->f16_used; i++) {
-    const eesen_b200_ctx::F16Entry &e = ctx->f16_slots[i];
-    if (e.ld != ld || P < e.base) continue;
-    const long off = (long)(P - e.base), ro = off / ld, co = off % ld;
-    if (ro + r > e.rows || co + c > e.cols || (co & 7)) continue;
-    *out = e.view;
-    out->hi = (const char *)e.view.hi + ((size_t)ro * e.ldd + co) * 2;
-    out->lo = (const char *)e.view.lo + ((size_t)ro * e.ldd + co) * 2;
-    return true;
-  }
-  for (int i = 0; i < eesen_b200_ctx::kActSlots; i++) {
-    const eesen_b200_ctx::ActPlanes &e = ctx->act[i];
-    if (!e.base || e.gen != ctx->act_gen || e.ld != ld || P < e.base) continue;
-    const long off = (long)(P - e.base), ro = off / ld, co = off % ld;
-    if (ro + r > e.rows || co + c > e.cols || (co & 7)) continue;
-    *out = e.view;
-    out->hi = (const char *)e.view.hi + ((size_t)ro * e.ldd + co) * 2;
-    out->lo = (const char *)e.view.lo + ((size_t)ro * e.ldd + co) * 2;
-    return true;
-  }
+  for (int i = 0; i < ctx->f16_used; i++)
+    if (ctx->f16_slots[i].find(P, r, c, ld, out)) return true;
+  for (int i = 0; i < eesen_b200_ctx::kActSlots; i++)
+    if (ctx->act[i].gen == ctx->act_gen && ctx->act[i].find(P, r, c, ld, out)) return true;
   return false;
+}
+
+// convert the whole matrix [rows x cols] (ld) and remember it: later products find sub-blocks by address
+// persist (only while a Net drives a training forward pass, ctx->act_enable): the planes go to a per-pass entry and stay
+// valid until the next forward pass -- the input weights Wx, which the dX product of the backward pass reads again
+static int f16_register(eesen_b200_ctx *ctx, const float *base, long rows, int cols, int ld, bool on_side = false,
+                        const unsigned *known_max = nullptr, bool persist = false) {
+  if (!ctx->f16x3 || ctx->gemm_prec != 0 || ctx->gemm_engine != 0 || !base || rows <= 0 || cols <= 0) return 0;
+  { eb::F16View have; if (f16_lookup(ctx, base, rows, cols, ld, &have)) return 0; }   // (e.g. planes the forward kernel wrote)
+  const bool act = persist && ctx->act_enable;
+  if (!act && ctx->f16_used >= eesen_b200_ctx::kF16Slots) return 0;   // (falls back to per-call conversion)
+  const int slot = act ? act_slot(ctx, base) : ctx->f16_used;
+  eesen_b200_ctx::PlaneEntry &e = act ? ctx->act[slot] : ctx->f16_slots[slot];
+  const int meta = act ? eesen_b200_ctx::kMetaAct + slot : eesen_b200_ctx::kMetaCall + slot;
+  int rc = convert_planes(ctx, e.planes, meta, base, rows, cols, ld, on_side, known_max, true, &e.view);
+  if (rc) return rc;
+  e.base = base; e.rows = rows; e.cols = cols; e.ld = ld; e.gen = act ? ctx->act_gen : 0;
+  if (!act) ctx->f16_used++;
+  return 0;
 }
 
 // planes for the layer output `out` [rows x cols] (ld) that the tcgen05 forward kernel is about to write (fixed scale 2^13)
 static int act_planes_for(eesen_b200_ctx *ctx, const float *out, long rows, int cols, int ld, eb::LstmFwdArgs *a) {
   if (!ctx->act_enable || !ctx->f16x3 || ctx->gemm_prec != 0 || ctx->gemm_engine != 0 || (cols & 7)) return 0;
-  int slot = -1;
-  for (int i = 0; i < eesen_b200_ctx::kActSlots; i++)
-    if (ctx->act[i].base == out) slot = i;
-  if (slot < 0) { slot = ctx->act_next; ctx->act_next = (ctx->act_next + 1) % eesen_b200_ctx::kActSlots; }
-  eesen_b200_ctx::ActPlanes &e = ctx->act[slot];
-  const size_t pb = eb::f16x2_plane_bytes(rows, cols);
-  void *pl = nullptr;
-  int rc = ctx->reserve(e.planes, 2 * pb + 256, &pl);
+  eesen_b200_ctx::PlaneEntry &e = ctx->act[act_slot(ctx, out)];
+  int rc = reserve_planes(ctx, e.planes, rows, cols, cols, &e.view);
   if (rc) return rc;
   if (!ctx->act_kexp) {
     unsigned *mx; int *kx;
-    if ((rc = f16_meta(ctx, eesen_b200_ctx::kF16Slots + 5, &mx, &kx))) return rc;
+    if ((rc = f16_meta(ctx, eesen_b200_ctx::kMetaK13, &mx, &kx))) return rc;
     static const int k13 = 13;
     if ((rc = ctx->check(cudaMemcpyAsync(kx, &k13, sizeof(int), cudaMemcpyHostToDevice, ctx->stream), "cudaMemcpyAsync"))) return rc;
     ctx->act_kexp = kx;
   }
-  e.base = out; e.rows = rows; e.cols = cols; e.ld = ld; e.ldd = cols; e.gen = ctx->act_gen;
-  e.view.hi = pl; e.view.lo = (char *)pl + ((pb + 255) & ~(size_t)255); e.view.ld = e.ldd; e.view.kexp = ctx->act_kexp;
-  a->out_hi = (void *)e.view.hi; a->out_lo = (void *)e.view.lo; a->ldh = e.ldd;
+  e.base = out; e.rows = rows; e.cols = cols; e.ld = ld; e.gen = ctx->act_gen; e.view.kexp = ctx->act_kexp;
+  a->out_hi = (void *)e.view.hi; a->out_lo = (void *)e.view.lo; a->ldh = e.view.ld;
   return 0;
 }
 
 // view of an operand: registered, or converted on the spot into the stream's temporary planes (which = 0 A, 1 B)
 static int f16_operand(eesen_b200_ctx *ctx, bool on_side, int which, const float *P, long r, int c, int ld, eb::F16View *out) {
   if (f16_lookup(ctx, P, r, c, ld, out)) return 0;
-  eesen_b200_ctx::Buf &b = ctx->f16_tmp[(on_side ? 2 : 0) + which];
-  const size_t pb = eb::f16x2_plane_bytes(r, c);
-  void *pl = nullptr;
-  int rc = ctx->reserve(b, 2 * pb + 256, &pl);
-  if (rc) return rc;
-  unsigned *mx; int *kx;
-  if ((rc = f16_meta(ctx, eesen_b200_ctx::kF16Slots + (on_side ? 2 : 0) + which, &mx, &kx))) return rc;
-  out->hi = pl; out->lo = (char *)pl + ((pb + 255) & ~(size_t)255); out->ld = (c + 7) & ~7; out->kexp = kx;
-  ctx->launches += 2;
-  return ctx->check(eb::convert_f16x2(on_side ? ctx->side : ctx->stream, ctx->num_sms, P, r, c, ld, (void *)out->hi,
-                                      (void *)out->lo, mx, kx), "convert_f16x2");
+  const int t = (on_side ? 2 : 0) + which;
+  return convert_planes(ctx, ctx->f16_tmp[t], eesen_b200_ctx::kMetaTmp + t, P, r, c, ld, on_side, nullptr, false, out);
 }
 
 static int do_gemm(eesen_b200_ctx *ctx, int ta, int tb, int M, int N, int K, float alpha, const float *A, int lda,
                    long sA, const float *B, int ldb, long sB, float beta, float *C, int ldc, long sC,
                    const float *bias, long sBias, int batch, bool on_side = false) {
   void *ws = nullptr;
+  int rc;
   cudaStream_t st = on_side ? ctx->side : ctx->stream;
   eesen_b200_ctx::Buf &gemm_ws = on_side ? ctx->gemm_ws_side : ctx->gemm_ws;
   eesen_b200_ctx::Buf &bf16_a = on_side ? ctx->bf16_a_side : ctx->bf16_a, &bf16_b = on_side ? ctx->bf16_b_side : ctx->bf16_b;
-  // tensor-core engine: tcgen05/TMEM/TMA (gemm_tc.cu) for every arithmetic mode -- kind::tf32 for fp32x3 / tf32,
-  // kind::f16 on bf16 copies of the operands for bf16 (BASELINE config 4); the warp-level mma.sync kernel
-  // (gemm.cu) is kept for EESEN_B200_GEMM_ENGINE=legacy (A/B measurements) and matrices TMA cannot address
-  if (ctx->gemm_engine == 0 && ctx->gemm_prec == 0 && ctx->f16x3 && !(ta && tb) && M > 0 && N > 0 && K > 0 &&
-      eb::gemm_tc_supported(ta, tb, M, N, K, A, 4, B, 4, 0)) {
-    // fp32-faithful arithmetic on the 16-bit tensor pipe: two fp16 planes per operand (registered whole-matrix
-    // conversions where the caller made them, else converted here), three kind::f16 MMAs per k-slice
-    size_t need_tc = eb::gemm_tc_workspace_bytes(M, N, K, ctx->num_sms);
-    if (need_tc) {
-      int rc = ctx->reserve(gemm_ws, need_tc, &ws);
-      if (rc) return rc;
-    }
-    const long ar = ta ? K : M, br = tb ? N : K;
-    const int ac = ta ? M : K, bc = tb ? K : N;
-    for (int b = 0; b < batch; b++) {
-      int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-      eb::F16View va, vb;
-      int rc;
-      if ((rc = f16_operand(ctx, on_side, 0, A + b * sA, ar, ac, lda, &va))) return rc;
-      if ((rc = f16_operand(ctx, on_side, 1, B + b * sB, br, bc, ldb, &vb))) return rc;
-      cudaError_t e = eb::gemm_tc16x3(st, ctx->num_sms, ta, tb, M, N, K, alpha, va, vb, beta, C + b * sC, ldc,
-                                      bias ? bias + b * sBias : nullptr, (float *)ws, ws ? gemm_ws.bytes : 0);
-      ctx->prof_end(pe);
-      ctx->launches += 1;
-      if ((rc = ctx->check(e, "gemm_tc16x3"))) return rc;
-    }
-    return 0;
+  // tensor-core engine: tcgen05/TMEM/TMA (gemm_tc.cu) for every arithmetic mode -- fp16x3: fp32-faithful arithmetic on
+  // the 16-bit tensor pipe, two fp16 planes per operand (registered whole-matrix conversions where the caller made them,
+  // else converted here), three kind::f16 MMAs per k-slice; bf16: kind::f16 on bf16 copies of the operands (BASELINE
+  // config 4); kind::tf32 for EESEN_B200_GEMM_FP32X3=tf32 and tf32.  The warp-level mma.sync kernel (gemm.cu) is kept
+  // for EESEN_B200_GEMM_ENGINE=legacy (A/B measurements) and matrices TMA cannot address.
+  enum { kLegacy, kF16x3, kBf16, kTf32 } eng = kLegacy;
+  const bool tc16 = !(ta && tb) && M > 0 && N > 0 && K > 0;
+  if (ctx->gemm_engine == 0) {
+    if (ctx->gemm_prec == 0 && ctx->f16x3 && tc16 && eb::gemm_tc_supported(ta, tb, M, N, K, A, 4, B, 4, 0))
+      eng = kF16x3;
+    else if (ctx->gemm_prec == 2 && tc16 && eb::gemm_tc_supported(ta, tb, M, N, K, A, 4, B, 4, 0))
+      eng = kBf16;
+    else if (eb::gemm_tc_supported(ta, tb, M, N, K, A, lda, B, ldb, ctx->gemm_prec) &&
+             (batch == 1 || ((sA & 3) == 0 && (sB & 3) == 0)))
+      eng = kTf32;
   }
-  if (ctx->gemm_engine == 0 && ctx->gemm_prec == 2 && !(ta && tb) && M > 0 && N > 0 && K > 0 &&
-      eb::gemm_tc_supported(ta, tb, M, N, K, A, 4, B, 4, 0)) {
-    size_t need_tc = eb::gemm_tc_workspace_bytes(M, N, K, ctx->num_sms);
-    if (need_tc) {
-      int rc = ctx->reserve(gemm_ws, need_tc, &ws);
-      if (rc) return rc;
-    }
-    // operands as stored: A [M x K] or [K x M], B [N x K] or [K x N]
-    const long ar = ta ? K : M, br = tb ? N : K;
-    const int ac = ta ? M : K, bc = tb ? K : N;
-    void *a16 = nullptr, *b16 = nullptr;
-    int rc;
+  if (eng == kLegacy) {
+    if (K >= 4096 && (rc = ctx->reserve(gemm_ws, eb::gemm_workspace_bytes(M, N, K, batch, ctx->num_sms), &ws))) return rc;
+    return launch(ctx, eesen_b200_ctx::kGemm, 1, "gemm", [&] {
+      return eb::gemm(st, ctx->num_sms, ta, tb, M, N, K, alpha, A, lda, sA, B, ldb, sB, beta, C, ldc, sC, bias, sBias,
+                      batch, ctx->gemm_prec, (float *)ws, ws ? gemm_ws.bytes : 0);
+    }, on_side);
+  }
+  const size_t need_tc = eb::gemm_tc_workspace_bytes(M, N, K, ctx->num_sms);
+  if (need_tc && (rc = ctx->reserve(gemm_ws, need_tc, &ws))) return rc;
+  const size_t ws_bytes = ws ? gemm_ws.bytes : 0;
+  // operands as stored: A [M x K] or [K x M], B [N x K] or [K x N]
+  const long ar = ta ? K : M, br = tb ? N : K;
+  const int ac = ta ? M : K, bc = tb ? K : N;
+  void *a16 = nullptr, *b16 = nullptr;
+  if (eng == kBf16) {
     if ((rc = ctx->reserve(bf16_a, eb::gemm_tc16_operand_bytes(ar, ac), &a16))) return rc;
     if ((rc = ctx->reserve(bf16_b, eb::gemm_tc16_operand_bytes(br, bc), &b16))) return rc;
-    for (int b = 0; b < batch; b++) {
-      int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-      cudaError_t e = cudaSuccess;
-      if (b == 0 || sA != 0) { e = eb::convert_bf16(st, ctx->num_sms, A + b * sA, ar, ac, lda, a16); ctx->launches += 1; }
-      if (e == cudaSuccess && (b == 0 || sB != 0)) { e = eb::convert_bf16(st, ctx->num_sms, B + b * sB, br, bc, ldb, b16); ctx->launches += 1; }
-      if (e == cudaSuccess)
-        e = eb::gemm_tc16(st, ctx->num_sms, ta, tb, M, N, K, alpha, a16, b16, beta, C + b * sC, ldc,
-                          bias ? bias + b * sBias : nullptr, (float *)ws, ws ? gemm_ws.bytes : 0);
-      ctx->prof_end(pe);
-      ctx->launches += 1;
-      if ((rc = ctx->check(e, "gemm_tc16"))) return rc;
-    }
-    return 0;
   }
-  if (ctx->gemm_engine == 0 && eb::gemm_tc_supported(ta, tb, M, N, K, A, lda, B, ldb, ctx->gemm_prec) &&
-      (batch == 1 || ((sA & 3) == 0 && (sB & 3) == 0))) {
-    size_t need_tc = eb::gemm_tc_workspace_bytes(M, N, K, ctx->num_sms);
-    if (need_tc) {
-      int rc = ctx->reserve(gemm_ws, need_tc, &ws);
-      if (rc) return rc;
+  for (int b = 0; b < batch; b++) {
+    const float *Ab = A + b * sA, *Bb = B + b * sB, *bb = bias ? bias + b * sBias : nullptr;
+    float *Cb = C + b * sC;
+    int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
+    cudaError_t e = cudaSuccess;
+    const char *what = "gemm_tc";
+    if (eng == kF16x3) {
+      eb::F16View va, vb;
+      if ((rc = f16_operand(ctx, on_side, 0, Ab, ar, ac, lda, &va))) return rc;
+      if ((rc = f16_operand(ctx, on_side, 1, Bb, br, bc, ldb, &vb))) return rc;
+      e = eb::gemm_tc16x3(st, ctx->num_sms, ta, tb, M, N, K, alpha, va, vb, beta, Cb, ldc, bb, (float *)ws, ws_bytes);
+      what = "gemm_tc16x3";
+    } else if (eng == kBf16) {
+      if (b == 0 || sA != 0) { e = eb::convert_bf16(st, ctx->num_sms, Ab, ar, ac, lda, a16); ctx->launches += 1; }
+      if (e == cudaSuccess && (b == 0 || sB != 0)) { e = eb::convert_bf16(st, ctx->num_sms, Bb, br, bc, ldb, b16); ctx->launches += 1; }
+      if (e == cudaSuccess) e = eb::gemm_tc16(st, ctx->num_sms, ta, tb, M, N, K, alpha, a16, b16, beta, Cb, ldc, bb, (float *)ws, ws_bytes);
+      what = "gemm_tc16";
+    } else {
+      e = eb::gemm_tc(st, ctx->num_sms, ta, tb, M, N, K, alpha, Ab, lda, Bb, ldb, beta, Cb, ldc, bb, ctx->gemm_prec,
+                      (float *)ws, ws_bytes);
     }
-    for (int b = 0; b < batch; b++) {
-      int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-      cudaError_t e = eb::gemm_tc(st, ctx->num_sms, ta, tb, M, N, K, alpha, A + b * sA, lda, B + b * sB, ldb,
-                                  beta, C + b * sC, ldc, bias ? bias + b * sBias : nullptr, ctx->gemm_prec,
-                                  (float *)ws, ws ? gemm_ws.bytes : 0);
-      ctx->prof_end(pe);
-      ctx->launches += 1;
-      int rc = ctx->check(e, "gemm_tc");
-      if (rc) return rc;
-    }
-    return 0;
+    ctx->prof_end(pe);
+    ctx->launches += 1;
+    if ((rc = ctx->check(e, what))) return rc;
   }
-  size_t need = eb::gemm_workspace_bytes(M, N, K, batch, ctx->num_sms);
-  if (K >= 4096) {
-    int rc = ctx->reserve(gemm_ws, need, &ws);
-    if (rc) return rc;
-  }
-  int pe = ctx->prof_begin(eesen_b200_ctx::kGemm, on_side);
-  cudaError_t e = eb::gemm(st, ctx->num_sms, ta, tb, M, N, K, alpha, A, lda, sA, B, ldb, sB, beta, C, ldc,
-                           sC, bias, sBias, batch, ctx->gemm_prec, (float *)ws, ws ? gemm_ws.bytes : 0);
-  ctx->prof_end(pe);
-  ctx->launches += 1;
-  return ctx->check(e, "gemm");
+  return 0;
 }
 
 int eesen_b200_gemm(eesen_b200_ctx *ctx, int transA, int transB, int M, int N, int K, float alpha, const float *A,
@@ -379,6 +329,20 @@ static int lstm_prepare(eesen_b200_ctx *ctx, int ndir, int pass, int S, int C, e
   return 0;
 }
 
+// the recurrent weights and peepholes of each direction for the kernels (ndir = 1: direction 0 in both), and the row
+// stride of Wx (0 in the params = dense)
+static int lstm_dir_params(eesen_b200_ctx *ctx, int ndir, int I, int C, const eesen_b200_bilstm_params *p,
+                           eb::LstmDirParams dp[2], int *ldwx) {
+  const int ldwm = p->ldwm > 0 ? p->ldwm : C;
+  *ldwx = p->ldwx > 0 ? p->ldwx : I;
+  if (*ldwx < I || ldwm < C) return ctx->fail(EESEN_B200_EINVAL, "ldwx / ldwm smaller than the matrix width");
+  for (int d = 0; d < 2; d++) {
+    const int q = d < ndir ? d : 0;
+    dp[d].wm = p->wm[q]; dp[d].ldwm = ldwm; dp[d].pi = p->pi[q]; dp[d].pf = p->pf[q]; dp[d].po = p->po[q];
+  }
+  return 0;
+}
+
 // ndir = 2: BiLstmParallel (gates [N x 8C], cell/out [N x 2C]); ndir = 1: LstmParallel, the forward cells
 // alone (gates [N x 4C], cell/out [N x C], index 0 of the parameter arrays) -- lstm-parallel-layer.h:47-113
 // is the forward-cell pass of bilstm-parallel-layer.h:97-150 line for line.
@@ -399,8 +363,9 @@ static int lstm_forward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I,
   // blocks are equally strided (they are in the Net arena), else two launches.
   long sW = ndir == 2 ? p->wx[1] - p->wx[0] : 0, sB = ndir == 2 ? p->bias[1] - p->bias[0] : 0;
   const int N = T * S, ldg = ndir * 4 * C;
-  const int ldwx = p->ldwx > 0 ? p->ldwx : I, ldwm = p->ldwm > 0 ? p->ldwm : C;
-  if (ldwx < I || ldwm < C) return ctx->fail(EESEN_B200_EINVAL, "ldwx / ldwm smaller than the matrix width");
+  eb::LstmFwdArgs a;
+  int ldwx;
+  if ((rc = lstm_dir_params(ctx, ndir, I, C, p, a.p, &ldwx))) return rc;
   // fp16x3: the layer input feeds the products of both directions -- one conversion
   ctx->join_side();
   ctx->f16_clear();
@@ -411,10 +376,10 @@ static int lstm_forward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I,
   // order the two directions consume G -- direction 0 from t = 0 upwards, direction 1 from t = T-1 downwards.  The
   // first kReady chunks run here, the others on the side stream next to the recurrent kernel, which checks
   // gflag[chunk] before the first read of a chunk.
-  const int kReady = ctx->fwd_ready_chunks;   // (EESEN_B200_FWD_READY, default 1: measured 14.86 vs 15.13 (2) vs 15.45 ms (3) per C2 step)
+  const int kReady = 1;   // (measured per C2 step: 14.86 ms at 1, 15.13 at 2, 15.45 at 3)
   int gchunk = 0, nchunks_g = 0;
   unsigned *gflags = nullptr;
-  if (plan.engine == 1 && chunk == S && ctx->overlap && ctx->stream_gemm && T >= 256) {
+  if (plan.engine == 1 && chunk == S && ctx->overlap && T >= 256) {
     gchunk = std::max(32, (T + 9) / 10);
     nchunks_g = (T + gchunk - 1) / gchunk;
     if (nchunks_g <= kReady || nchunks_g > 64) nchunks_g = 0;
@@ -437,10 +402,9 @@ static int lstm_forward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I,
                      gates + r0 * ldg + (size_t)d * 4 * C, ldg, 0, p->bias[d], 0, 1, on_side);
         if (rc) return rc;
       }
-      if (on_side) {
-        ctx->launches += 1;
-        if ((rc = ctx->check(eb::lstm_set_flag(ctx->side, gflags + ci, ctx->gepoch), "lstm_set_flag"))) return rc;
-      }
+      if (on_side && (rc = launch(ctx, kUntimed, 1, "lstm_set_flag",
+                                  [&] { return eb::lstm_set_flag(ctx->side, gflags + ci, ctx->gepoch); })))
+        return rc;
     }
   } else if (ndir == 2 && sW > 0 && (sW & 3) == 0 && sB > 0) {
     rc = do_gemm(ctx, 0, 1, N, 4 * C, I, 1.f, x, ldx, 0, p->wx[0], ldwx, sW, 0.f, gates, ldg, 4 * C, p->bias[0], sB, 2);
@@ -452,29 +416,20 @@ static int lstm_forward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I,
       if (rc) return rc;
     }
   }
-  eb::LstmFwdArgs a;
   a.T = T; a.S = S; a.C = C; a.len = d_len;
   a.G = gates; a.ldg = ldg;
   a.cell = cell; a.ldc = ndir * C;
   a.out = out; a.ldo = ldo;
-  for (int d = 0; d < 2; d++) {
-    const int q = d < ndir ? d : 0;
-    a.p[d].wm = p->wm[q]; a.p[d].ldwm = ldwm; a.p[d].pi = p->pi[q]; a.p[d].pf = p->pf[q]; a.p[d].po = p->po[q];
-  }
   a.xbuf = xbuf;
   a.precision = ctx->rec_prec;
   a.drop = drop; a.rmask = rmask; a.ldr = ldr; a.rmask_per_step = per_step;
-  { const char *tn = getenv("EESEN_B200_TUNE"); a.tune = tn ? atoi(tn) : 0; }
   if (plan.engine == 1 && (rc = act_planes_for(ctx, out, N, ndir * C, ldo, &a))) return rc;
   if (nchunks_g) { a.gflag = gflags; a.gepoch = ctx->gepoch; a.gchunk = gchunk; a.gready = kReady; }
   for (int s0 = 0; s0 < S; s0 += chunk) {
     a.s_begin = s0;
     a.s_count = std::min(chunk, S - s0);
-    ctx->launches += 1;
-    int pe = ctx->prof_begin(eesen_b200_ctx::kLstmFwd);
-    cudaError_t le = eb::lstm_forward(ctx->stream, plan, a);
-    ctx->prof_end(pe);
-    if ((rc = ctx->check(le, "lstm_forward"))) return rc;
+    if ((rc = launch(ctx, eesen_b200_ctx::kLstmFwd, 1, "lstm_forward", [&] { return eb::lstm_forward(ctx->stream, plan, a); })))
+      return rc;
   }
   return 0;
 }
@@ -502,21 +457,15 @@ int eesen_b200_bilstm_backward_dropout(eesen_b200_ctx *ctx, int T, int S, int I,
 int eesen_b200_mul_elements(eesen_b200_ctx *ctx, int N, int cols, const float *a, int lda, const float *b, int ldb,
                             float *out, int ldo) {
   if (!ctx || !a || !b || !out || N < 0 || cols < 1) return EESEN_B200_EINVAL;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kMisc);
-  cudaError_t e = eb::mul_elements(ctx->stream, ctx->num_sms, N, cols, a, lda, b, ldb, out, ldo);
-  ctx->prof_end(pe);
-  return ctx->check(e, "mul_elements");
+  return launch(ctx, eesen_b200_ctx::kMisc, 1, "mul_elements",
+                [&] { return eb::mul_elements(ctx->stream, ctx->num_sms, N, cols, a, lda, b, ldb, out, ldo); });
 }
 
 int eesen_b200_dropout_mask(eesen_b200_ctx *ctx, int rows, int cols, float *d_mask, int ld, float p, int per_col,
                             unsigned long long seed, unsigned long long stream) {
   if (!ctx || !d_mask || rows < 0 || cols < 1 || ld < cols || !(p >= 0.f && p < 1.f)) return EESEN_B200_EINVAL;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kMisc);
-  cudaError_t e = eb::dropout_mask(ctx->stream, ctx->num_sms, rows, cols, d_mask, ld, p, per_col, seed, stream);
-  ctx->prof_end(pe);
-  return ctx->check(e, "dropout_mask");
+  return launch(ctx, eesen_b200_ctx::kMisc, 1, "dropout_mask",
+                [&] { return eb::dropout_mask(ctx->stream, ctx->num_sms, rows, cols, d_mask, ld, p, per_col, seed, stream); });
 }
 
 int eesen_b200_lstm_forward(eesen_b200_ctx *ctx, int T, int S, int I, int C, const float *x, int ldx,
@@ -539,51 +488,34 @@ static int lstm_backward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I
   if (rc) return rc;
   const int nchunks = (S + chunk - 1) / chunk;
   const int ldg = ndir * 4 * C;
-  const int ldwx = p->ldwx > 0 ? p->ldwx : I, ldwm = p->ldwm > 0 ? p->ldwm : C;
-  const int gldwx = gr->ldwx > 0 ? gr->ldwx : I, gldwm = gr->ldwm > 0 ? gr->ldwm : C;
-  if (ldwx < I || ldwm < C || gldwx < I || gldwm < C)
-    return ctx->fail(EESEN_B200_EINVAL, "ldwx / ldwm smaller than the matrix width");
   eb::LstmBwdArgs a;
+  int ldwx;
+  if ((rc = lstm_dir_params(ctx, ndir, I, C, p, a.p, &ldwx))) return rc;
+  const int gldwx = gr->ldwx > 0 ? gr->ldwx : I, gldwm = gr->ldwm > 0 ? gr->ldwm : C;
+  if (gldwx < I || gldwm < C) return ctx->fail(EESEN_B200_EINVAL, "ldwx / ldwm smaller than the matrix width");
   a.T = T; a.S = S; a.C = C;
   a.G = gates; a.ldg = ldg;
   a.cell = cell; a.ldc = ndir * C;
   a.dout = dout; a.ldd = ldd;
   a.DG = dgates; a.lddg = ldg;
-  for (int d = 0; d < 2; d++) {
-    const int q = d < ndir ? d : 0;
-    a.p[d].wm = p->wm[q]; a.p[d].ldwm = ldwm; a.p[d].pi = p->pi[q]; a.p[d].pf = p->pf[q]; a.p[d].po = p->po[q];
-  }
   a.pbuf = pbuf; a.gsum = gsum;
   a.precision = ctx->rec_prec;
   a.drop = drop; a.rmask = rmask; a.ldr = ldr; a.rmask_per_step = per_step;
-  { const char *tn = getenv("EESEN_B200_TUNE"); a.tune = tn ? atoi(tn) : 0; }
-  // dout may be the dX the previous call is still streaming on the side stream (ctx->dxs): the tcgen05 kernel reads it
-  // chunk pair by chunk pair behind flags; any other consumer waits for all of it first
-  if (ctx->dxs.active) {
-    const eesen_b200_ctx::DxStream &dxs = ctx->dxs;
-    if (dout == dxs.ptr && ldd == dxs.ld && T == dxs.T && S == dxs.S && plan.engine == 1 && chunk == S) {
-      a.dflag = dxs.flags; a.depoch = dxs.epoch; a.dchunk = dxs.chunk; a.dnck = dxs.nck; a.dready = dxs.ready;
-    } else {
-      ctx->join_side();
-    }
-    ctx->dxs.active = false;
-  }
   // fp16x3: the layer input and m feed the weight-gradient products; they are forward activations, so their planes are
   // made on the side stream (behind the weight-gradient products of the layer above, which still read the previous
   // planes) WHILE the recurrent kernel below runs.  d(gates) and Wx follow on `stream` behind the kernel.
   const int N = T * S;
   const bool sd = ctx->overlap != 0;
-  const bool early = sd && ctx->early_conv;
   ctx->f16_clear();
   // max |DG| comes out of the tcgen05 kernel itself (a.dgmax): the conversion of DG below needs no scan of its own
   unsigned *dgmax = nullptr;
   if (plan.engine == 1 && ctx->f16x3 && ctx->gemm_prec == 0 && ctx->gemm_engine == 0) {
     int *unused_k;
-    if ((rc = f16_meta(ctx, eesen_b200_ctx::kF16Slots + 4, &dgmax, &unused_k))) return rc;
+    if ((rc = f16_meta(ctx, eesen_b200_ctx::kMetaDgmax, &dgmax, &unused_k))) return rc;
     if ((rc = ctx->check(cudaMemsetAsync(dgmax, 0, sizeof(unsigned), ctx->stream), "cudaMemsetAsync"))) return rc;
     a.dgmax = dgmax;
   }
-  if (early) {
+  if (sd) {
     ctx->fork_side();
     if ((rc = f16_register(ctx, x, N, I, ldx, true))) return rc;
     if (T > 1 && (rc = f16_register(ctx, out, N, ndir * C, ldo, true))) return rc;
@@ -592,87 +524,36 @@ static int lstm_backward_impl(eesen_b200_ctx *ctx, int ndir, int T, int S, int I
     a.s_begin = ci * chunk;
     a.s_count = std::min(chunk, S - a.s_begin);
     a.gsum = gsum + (size_t)ci * plan.gsum_floats;
-    ctx->launches += 1;
-    int pe = ctx->prof_begin(eesen_b200_ctx::kLstmBwd);
-    cudaError_t le = eb::lstm_backward(ctx->stream, plan, a);
-    ctx->prof_end(pe);
-    if ((rc = ctx->check(le, "lstm_backward"))) return rc;
+    if ((rc = launch(ctx, eesen_b200_ctx::kLstmBwd, 1, "lstm_backward", [&] { return eb::lstm_backward(ctx->stream, plan, a); })))
+      return rc;
   }
-  for (int d = 0; d < ndir; d++) {
-    ctx->launches += 1;
-    int pe = ctx->prof_begin(eesen_b200_ctx::kMisc);
-    cudaError_t le = eb::lstm_reduce_gsum(ctx->stream, plan, C, gsum, nchunks, gr->bias[d], gr->pi[d], gr->pf[d], gr->po[d], d);
-    ctx->prof_end(pe);
-    if ((rc = ctx->check(le, "lstm_reduce_gsum"))) return rc;
-  }
+  for (int d = 0; d < ndir; d++)
+    if ((rc = launch(ctx, eesen_b200_ctx::kMisc, 1, "lstm_reduce_gsum", [&] {
+           return eb::lstm_reduce_gsum(ctx->stream, plan, C, gsum, nchunks, gr->bias[d], gr->pi[d], gr->pf[d], gr->po[d], d);
+         })))
+      return rc;
   // fp16x3: d(gates), the layer input, m and Wx each feed several of the products below -- one conversion each.
   // The planes of the previous layer call may still be read by its weight-gradient products on the side stream:
   // they have had the whole recurrent kernel above to finish, now they are waited for.
   ctx->join_side();
-  if (!early) {
+  if (!sd) {
     if ((rc = f16_register(ctx, x, N, I, ldx))) return rc;
     if (T > 1 && (rc = f16_register(ctx, out, N, ndir * C, ldo))) return rc;
   }
   if ((rc = f16_register(ctx, dgates, N, ndir * 4 * C, ldg, false, dgmax))) return rc;
-  if (dx)
+  if (dx) {
     for (int d = 0; d < ndir; d++)
       if ((rc = f16_register(ctx, p->wx[d], 4 * C, I, ldwx))) return rc;
-  // dx = DG_fw * Wx_fw + DG_bw * Wx_bw   (:502 beta=0, :593 beta=1), rows [r0, r0 + nr)
-  auto dx_rows = [&](long r0, long nr, bool on_side) -> int {
-    for (int d = 0; d < ndir; d++) {
-      int rc2 = do_gemm(ctx, 0, 0, (int)nr, I, 4 * C, 1.f, dgates + (size_t)r0 * ldg + (size_t)d * 4 * C, ldg, 0, p->wx[d], ldwx, 0,
-                        d == 0 ? 0.f : 1.f, dx + (size_t)r0 * lddx, lddx, 0, nullptr, 0, 1, on_side);
-      if (rc2) return rc2;
-    }
-    return 0;
-  };
-  // Streamed (see context.h:DxStream): Net announced that dx goes straight into the recurrent backward of the layer
-  // below.  Time chunks of g positions; pair ci = chunk ci and chunk nck-1-ci -- direction 0 of the layer below starts at
-  // t = T-1, direction 1 at t = 0.  Pair 0 here, the others on the side stream in front of the weight-gradient products.
-  bool stream_dx = false;
-  int dg = 0, dnck = 0, dnpairs = 0;
-  if (dx && sd && ctx->dx_stream_hint && ctx->stream_dx && ctx->stream_gemm && plan.engine == 1 && chunk == S && T >= 256) {
-    dg = std::max(16, (T + 9) / 10);
-    dnck = (T + dg - 1) / dg;
-    dnpairs = (dnck + 1) / 2;
-    stream_dx = dnpairs > ctx->dx_ready_pairs && dnpairs <= 64;
-  }
-  unsigned *dflags = nullptr;
-  if (stream_dx) {
-    void *df = nullptr;
-    const bool fresh = ctx->lstm_dflags.bytes == 0;
-    if ((rc = ctx->reserve(ctx->lstm_dflags, 64 * sizeof(unsigned), &df))) return rc;
-    dflags = (unsigned *)df;
-    if (fresh && (rc = ctx->check(cudaMemsetAsync(df, 0, 64 * sizeof(unsigned), ctx->stream), "cudaMemsetAsync"))) return rc;
-    ctx->depoch += 1;
-    if (ctx->depoch == 0u) ctx->depoch = 1;
-  }
-  auto dx_pair = [&](int ci, bool on_side) -> int {
-    const int k1 = ci, k2 = dnck - 1 - ci;
-    int rc2 = dx_rows((long)k1 * dg * S, (long)std::min(dg, T - k1 * dg) * S, on_side);
-    if (!rc2 && k2 > k1) rc2 = dx_rows((long)k2 * dg * S, (long)std::min(dg, T - k2 * dg) * S, on_side);
-    return rc2;
-  };
-  if (dx && !stream_dx) {
-    if ((rc = dx_rows(0, N, false))) return rc;
-  } else if (dx) {
-    for (int ci = 0; ci < ctx->dx_ready_pairs; ci++)
-      if ((rc = dx_pair(ci, false))) return rc;
+    // dx = DG_fw * Wx_fw + DG_bw * Wx_bw   (:502 beta=0, :593 beta=1)
+    for (int d = 0; d < ndir; d++)
+      if ((rc = do_gemm(ctx, 0, 0, N, I, 4 * C, 1.f, dgates + (size_t)d * 4 * C, ldg, 0, p->wx[d], ldwx, 0,
+                        d == 0 ? 0.f : 1.f, dx, lddx, 0, nullptr, 0, 1)))
+        return rc;
   }
   // The weight-gradient products below are consumed only by the all-reduce / update at the end of the step: they go
   // to the side stream (forked here, after the recurrent kernel and the bias / peephole sums) and overlap with the
   // dX product above and with the recurrent backward of the layer below.
   if (sd) ctx->fork_side();
-  if (stream_dx) {
-    for (int ci = ctx->dx_ready_pairs; ci < dnpairs; ci++) {
-      if ((rc = dx_pair(ci, true))) return rc;
-      ctx->launches += 1;
-      if ((rc = ctx->check(eb::lstm_set_flag(ctx->side, dflags + ci, ctx->depoch), "lstm_set_flag"))) return rc;
-    }
-    eesen_b200_ctx::DxStream &dxs = ctx->dxs;
-    dxs.active = true; dxs.ptr = dx; dxs.ld = lddx; dxs.T = T; dxs.S = S; dxs.chunk = dg; dxs.nck = dnck; dxs.ready = ctx->dx_ready_pairs;
-    dxs.flags = dflags; dxs.epoch = ctx->depoch;
-  }
   long sGW = ndir == 2 ? gr->wx[1] - gr->wx[0] : 0, sGM = ndir == 2 ? gr->wm[1] - gr->wm[0] : 0;
   bool batched = ndir == 2 && sGW > 0 && (sGW & 3) == 0 && sGM > 0 && (sGM & 3) == 0;
   // Wx grad = DG^T * x   (:505 / :596), both directions batched
@@ -745,11 +626,9 @@ int eesen_b200_affine_backward(eesen_b200_ctx *ctx, int N, int D, int K, const f
   if (db) {
     void *ws = nullptr;
     if ((rc = ctx->reserve(ctx->colsum_ws, eb::col_sum_ws_floats(K, ctx->num_sms) * sizeof(float), &ws))) return rc;
-    ctx->launches += 2;
-    int pe = ctx->prof_begin(eesen_b200_ctx::kMisc);
-    cudaError_t ce = eb::col_sum(ctx->stream, ctx->num_sms, N, K, diff, lddiff, db, (float *)ws);
-    ctx->prof_end(pe);
-    if ((rc = ctx->check(ce, "col_sum"))) return rc;
+    if ((rc = launch(ctx, eesen_b200_ctx::kMisc, 2, "col_sum",
+                     [&] { return eb::col_sum(ctx->stream, ctx->num_sms, N, K, diff, lddiff, db, (float *)ws); })))
+      return rc;
   }
   return 0;
 }
@@ -757,31 +636,23 @@ int eesen_b200_affine_backward(eesen_b200_ctx *ctx, int N, int D, int K, const f
 int eesen_b200_softmax(eesen_b200_ctx *ctx, int N, int K, const float *logits, int ld, float *probs, int ldp,
                        int *d_argmax) {
   if (!ctx || !logits || !probs) return EESEN_B200_EINVAL;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kSoftmax);
-  cudaError_t e = eb::softmax_rows(ctx->stream, N, K, logits, ld, probs, ldp, d_argmax);
-  ctx->prof_end(pe);
-  return ctx->check(e, "softmax_rows");
+  return launch(ctx, eesen_b200_ctx::kSoftmax, 1, "softmax_rows",
+                [&] { return eb::softmax_rows(ctx->stream, N, K, logits, ld, probs, ldp, d_argmax); });
 }
 
 int eesen_b200_row_argmax(eesen_b200_ctx *ctx, int N, int K, const float *x, int ld, int *d_argmax) {
   if (!ctx || !x || !d_argmax) return EESEN_B200_EINVAL;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kSoftmax);
-  cudaError_t e = eb::row_argmax(ctx->stream, N, K, x, ld, d_argmax);
-  ctx->prof_end(pe);
-  return ctx->check(e, "row_argmax");
+  return launch(ctx, eesen_b200_ctx::kSoftmax, 1, "row_argmax",
+                [&] { return eb::row_argmax(ctx->stream, N, K, x, ld, d_argmax); });
 }
 
 int eesen_b200_loglik(eesen_b200_ctx *ctx, int N, int K, float *y, int ld, int apply_log, const float *d_log_prior,
                       float prior_scale) {
   if (!ctx || !y || N < 0 || K < 1 || ld < K) return EESEN_B200_EINVAL;
   if (!apply_log && !d_log_prior) return 0;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kSoftmax);
-  cudaError_t e = eb::loglik_rows(ctx->stream, ctx->num_sms, N, K, y, ld, apply_log, d_log_prior, prior_scale);
-  ctx->prof_end(pe);
-  return ctx->check(e, "loglik_rows");
+  return launch(ctx, eesen_b200_ctx::kSoftmax, 1, "loglik_rows", [&] {
+    return eb::loglik_rows(ctx->stream, ctx->num_sms, N, K, y, ld, apply_log, d_log_prior, prior_scale);
+  });
 }
 
 int eesen_b200_ctc_eval(eesen_b200_ctx *ctx, int T, int S, int K, int max_lab, const int *d_len, const int *d_labels,
@@ -791,12 +662,9 @@ int eesen_b200_ctc_eval(eesen_b200_ctx *ctx, int T, int S, int K, int max_lab, c
   void *ws = nullptr;
   int rc = ctx->reserve(ctx->ctc_ws, eb::ctc_workspace_floats(T, S, max_lab) * sizeof(float), &ws);
   if (rc) return rc;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kCtc);
-  cudaError_t e = eb::ctc_eval(ctx->stream, T, S, K, max_lab, d_len, d_labels, d_lab_len, probs, ldp, pzx, diff, ldd,
-                               (float *)ws);
-  ctx->prof_end(pe);
-  return ctx->check(e, "ctc_eval");
+  return launch(ctx, eesen_b200_ctx::kCtc, 1, "ctc_eval", [&] {
+    return eb::ctc_eval(ctx->stream, T, S, K, max_lab, d_len, d_labels, d_lab_len, probs, ldp, pzx, diff, ldd, (float *)ws);
+  });
 }
 
 int eesen_b200_ce_eval(eesen_b200_ctx *ctx, int T, int S, int K, const int *d_len, const float *probs, int ldp,
@@ -807,11 +675,9 @@ int eesen_b200_ce_eval(eesen_b200_ctx *ctx, int T, int S, int K, const int *d_le
   void *ws = nullptr;
   int rc = ctx->reserve(ctx->ce_ws, eb::ce_workspace_bytes(T, S, ctx->num_sms), &ws);
   if (rc) return rc;
-  ctx->launches += 2;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kSoftmax);
-  cudaError_t e = eb::ce_eval(ctx->stream, ctx->num_sms, T, S, K, d_len, probs, ldp, d_targets, diff, ldd, d_stats, ws);
-  ctx->prof_end(pe);
-  return ctx->check(e, "ce_eval");
+  return launch(ctx, eesen_b200_ctx::kSoftmax, 2, "ce_eval", [&] {
+    return eb::ce_eval(ctx->stream, ctx->num_sms, T, S, K, d_len, probs, ldp, d_targets, diff, ldd, d_stats, ws);
+  });
 }
 
 int eesen_b200_check_finite(eesen_b200_ctx *ctx, const float *d_x, int64_t n, int *flags) {
@@ -820,11 +686,9 @@ int eesen_b200_check_finite(eesen_b200_ctx *ctx, const float *d_x, int64_t n, in
   void *d = nullptr;
   int rc = ctx->reserve(ctx->flag_buf, 64, &d);
   if (rc) return rc;
-  ctx->launches += 1;
-  int pe = ctx->prof_begin(eesen_b200_ctx::kMisc);
-  cudaError_t e = eb::check_finite(ctx->stream, ctx->num_sms, d_x, (long)n, (int *)d);
-  ctx->prof_end(pe);
-  if ((rc = ctx->check(e, "check_finite"))) return rc;
+  if ((rc = launch(ctx, eesen_b200_ctx::kMisc, 1, "check_finite",
+                   [&] { return eb::check_finite(ctx->stream, ctx->num_sms, d_x, (long)n, (int *)d); })))
+    return rc;
   CTX_CHECK(cudaMemcpyAsync(flags, d, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream), "memcpy(flags)");
   CTX_CHECK(cudaStreamSynchronize(ctx->stream), "sync(flags)");
   return 0;
@@ -845,9 +709,9 @@ int eesen_b200_sgd_update(eesen_b200_ctx *ctx, float *w, float *corr, const floa
   // synchronous small copy: the host vector dies at return
   CTX_CHECK(cudaMemcpyAsync(d, h.data(), sizeof(eb::SgdSegment) * nseg, cudaMemcpyHostToDevice, ctx->stream), "memcpy(segments)");
   CTX_CHECK(cudaStreamSynchronize(ctx->stream), "sync(segments)");
-  ctx->launches += 1;
-  return ctx->check(eb::sgd_momentum_clip(ctx->stream, ctx->num_sms, w, corr, grad, momentum, (eb::SgdSegment *)d, nseg,
-                                          (long)n), "sgd_momentum_clip");
+  return launch(ctx, kUntimed, 1, "sgd_momentum_clip", [&] {
+    return eb::sgd_momentum_clip(ctx->stream, ctx->num_sms, w, corr, grad, momentum, (eb::SgdSegment *)d, nseg, (long)n);
+  });
 }
 
 // ------------------------------------------------------------------------------------ NCCL (dlopen)

@@ -33,41 +33,49 @@ struct eesen_b200_ctx {
   Buf decode_ws;
   Buf ce_ws;   // per-CTA partial sums of the cross-entropy statistics
 
-  // fp16x3 arithmetic (gemm_prec 0 on the 16-bit tensor pipe): converted operand planes.  Whole matrices that feed
-  // several products of one layer call (d(gates), the layer input, m, Wx) are converted ONCE and registered here;
-  // do_gemm finds sub-blocks of them by address.  Entries live until the next f16_clear().
-  struct F16Entry {
+  // fp16x3 arithmetic (gemm_prec 0 on the 16-bit tensor pipe): converted operand planes of whole matrices that feed
+  // several products; do_gemm finds sub-blocks of them by address.
+  struct PlaneEntry {
     const float *base = nullptr;
     long rows = 0;
-    int cols = 0, ld = 0, ldd = 0;
+    int cols = 0, ld = 0;
+    unsigned gen = 0;    // (act) the forward pass that made the planes
     Buf planes;          // hi plane, then lo plane
     eb::F16View view;
+    // the [r x c] block at P with leading dimension ld_, if it lies in this matrix on an 8-column boundary
+    bool find(const float *P, long r, int c, int ld_, eb::F16View *out) const {
+      if (!base || ld_ != ld || P < base) return false;
+      const long off = (long)(P - base), ro = off / ld, co = off % ld;
+      if (ro + r > rows || co + c > cols || (co & 7)) return false;
+      *out = view;
+      out->hi = (const char *)view.hi + ((size_t)ro * view.ld + co) * 2;
+      out->lo = (const char *)view.lo + ((size_t)ro * view.ld + co) * 2;
+      return true;
+    }
   };
+  // Per layer call: d(gates), the layer input, m, Wx are converted ONCE and registered here; they live until the next
+  // f16_clear().
   enum { kF16Slots = 6 };
-  F16Entry f16_slots[kF16Slots];
+  PlaneEntry f16_slots[kF16Slots];
   int f16_used = 0;
-  Buf f16_meta;          // per slot + per temp operand: {unsigned max scratch, int kexp}
+  void f16_clear() { f16_used = 0; }
   Buf f16_tmp[4];        // ad-hoc operands: [0] A / [1] B on `stream`, [2] A / [3] B on the side stream
   int f16x3 = 1;         // EESEN_B200_GEMM_FP32X3=tf32 : keep the kind::tf32 3-term split (A/B measurements)
-  void f16_clear() { f16_used = 0; }
-  // Planes of layer outputs written by the recurrent forward kernel itself (LstmFwdArgs::out_hi): they outlive
-  // f16_clear() -- the next layer's input product, and both weight-gradient products of the backward pass, find them by
-  // address and convert nothing.  Only while a Net drives the step (act_enable, set by Net::Propagate in training mode;
-  // act_gen: one generation per forward pass, older entries are dead), so that callers of the level-1 operators who reuse
-  // buffers never meet planes of other data.
-  struct ActPlanes {
-    const float *base = nullptr;
-    long rows = 0;
-    int cols = 0, ld = 0, ldd = 0;
-    unsigned gen = 0;
-    Buf planes;
-    eb::F16View view;
-  };
+  // Per forward pass: planes of layer outputs written by the recurrent forward kernel itself (LstmFwdArgs::out_hi), and
+  // of the input weights Wx, outlive f16_clear() -- the next layer's input product, and the products of the backward
+  // pass, find them by address and convert nothing.  Only while a Net drives the step (act_enable, set by
+  // Net::Propagate in training mode; act_gen: one generation per forward pass, older entries are dead), so that callers
+  // of the level-1 operators who reuse buffers never meet planes of other data.
   enum { kActSlots = 32 };
-  ActPlanes act[kActSlots];
+  PlaneEntry act[kActSlots];
   int act_next = 0, act_enable = 0;
   unsigned act_gen = 1;
   int *act_kexp = nullptr;   // device: the constant 13
+  // f16_meta: 4096 bytes of 8-byte device records {unsigned max scratch, int kexp}, indexed from these bases: per-call
+  // entries, the four temporary operands (as f16_tmp), max |d(gates)| of the recurrent backward kernel, act_kexp,
+  // per-pass entries
+  enum { kMetaCall = 0, kMetaTmp = kF16Slots, kMetaDgmax = kMetaTmp + 4, kMetaK13 = kMetaTmp + 5, kMetaAct = kMetaTmp + 8 };
+  Buf f16_meta;
 
   // Side stream (lower priority): work nothing on the critical path waits for -- the weight-gradient products of
   // layer l and the all-reduce of its gradient block run here while `stream` carries dX and the recurrent backward
@@ -79,30 +87,9 @@ struct eesen_b200_ctx {
   bool side_pending = false;
   int overlap = 1;   // EESEN_B200_OVERLAP=0: everything on `stream` (A/B measurements)
   // Streamed input product of the recurrent forward pass: x*Wx^T is cut into chunks of time steps in the order the
-  // two directions consume them; the first chunks run on `stream`, the rest on the side stream WHILE the recurrent
-  // kernel runs (it checks a per-chunk flag before it reads a chunk).  EESEN_B200_STREAM_GEMM=0 turns it off.
-  int stream_gemm = 1;
-  int fwd_ready_chunks = 1;   // chunks of the streamed input product computed on `stream` before the kernel starts
+  // two directions consume them; the first chunk runs on `stream`, the rest on the side stream WHILE the recurrent
+  // kernel runs (it checks a per-chunk flag before it reads a chunk).
   unsigned gepoch = 0;
-  // Streamed dX of the recurrent backward pass (the same idea, other direction): when the caller (Net) says that the
-  // in_diff of this layer goes straight into the recurrent backward of the layer below (dx_stream_hint), DG*Wx is cut
-  // into pairs of time chunks -- the two ends of the sequence first, where the two directions of the layer below
-  // start -- the first pair runs on `stream`, the others on the side stream while the recurrent kernel of the layer
-  // below already runs; it checks dflags[pair] before it reads a chunk of its dout.  `dxs` describes the matrix being
-  // streamed; the next recurrent backward call matches it by address (anything else first joins the side stream).
-  int dx_stream_hint = 0;
-  int stream_dx = 0;       // EESEN_B200_STREAM_DX=1 turns the streamed dX on (measured: the side stream has no room for it)
-  int dx_ready_pairs = 1;  // EESEN_B200_DX_READY: chunk pairs computed on `stream` before the layer below starts
-  int early_conv = 1;      // EESEN_B200_EARLY_CONV=0: planes of x / m made behind the recurrent backward kernel, on `stream`
-  struct DxStream {
-    bool active = false;
-    const float *ptr = nullptr;
-    int ld = 0, T = 0, S = 0, chunk = 0, nck = 0, ready = 0;
-    unsigned *flags = nullptr;
-    unsigned epoch = 0;
-  } dxs;
-  Buf lstm_dflags;
-  unsigned depoch = 0;
   void fork_side() {
     cudaEventRecord(ev_fork, stream);
     cudaStreamWaitEvent(side, ev_fork, 0);

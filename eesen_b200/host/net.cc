@@ -1041,10 +1041,7 @@ void Net::BackpropagateLayers(const CuMatrixBase<BaseFloat> *out_diff, CuMatrix<
   for (int32 i = NumLayers() - 1; i >= 0; i--) {
     if (out_diff) {
       layers_[i]->need_in_diff_ = (i > 0) || (in_diff != NULL);
-      // the in_diff of a recurrent layer may be streamed into the recurrent backward of the layer below (DxStream)
-      ctx_->dx_stream_hint = (i > 0 && layers_[i - 1]->TakesOutDiffAsIs()) ? 1 : 0;
       layers_[i]->Backpropagate(propagate_buf_[i], propagate_buf_[i + 1], *diff, &backpropagate_buf_[i]);
-      ctx_->dx_stream_hint = 0;
       diff = &backpropagate_buf_[i];
     }
     if (nranks > 1 && layer_offset_[i] >= 0) {

@@ -109,9 +109,6 @@ class Layer {
   static const char *TypeToMarker(LayerType t);
   static LayerType MarkerToType(const std::string &s);
   virtual std::string Info() const { return ""; }
-  // true when BackpropagateFnc hands out_diff to the recurrent backward kernel unchanged (no forward-dropout mask in
-  // between): Net then lets the layer above stream its in_diff (context.h:DxStream)
-  virtual bool TakesOutDiffAsIs() const { return false; }
 
  protected:
   friend class Net;
@@ -149,7 +146,6 @@ class BiLstmParallel : public TrainableLayer {
  public:
   BiLstmParallel(int32 in, int32 out) : TrainableLayer(in, out), cell_dim_(out / 2) {}
   LayerType GetType() const { return l_BiLstm_Parallel; }
-  bool TakesOutDiffAsIs() const { return !apply_fwd_; }
   LayerType GetTypeNonParal() const { return l_BiLstm; }
   void SetSeqLengths(std::vector<int> &sequence_lengths);
   int64 NumParams() const;
@@ -220,7 +216,6 @@ class LstmParallel : public TrainableLayer {
   LstmParallel(int32 in, int32 out, bool nonparallel = false)
       : TrainableLayer(in, out), cell_dim_(out), nonparallel_(nonparallel) {}
   LayerType GetType() const { return nonparallel_ ? l_Lstm : l_Lstm_Parallel; }
-  bool TakesOutDiffAsIs() const { return true; }
   LayerType GetTypeNonParal() const { return l_Lstm; }
   void SetSeqLengths(std::vector<int> &sequence_lengths) { num_streams_ = (int32)sequence_lengths.size(); }
   int64 NumParams() const { int64 C = cell_dim_, I = input_dim_; return 4 * C * I + 4 * C * C + 4 * C + 3 * C; }
